@@ -3,8 +3,11 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N ...            # the reference algorithm on the host CPU cores (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results to DIR/*.npy
 
-A "step" is one pass of the whole PicketFence pipeline over one batch of synthetic frames (config.workload).
+A "step" is one pass of the whole PicketFence pipeline over one batch of synthetic frames (config.workload); every PicketFence leg
+below times exactly K steps.  The frames are generated from fixed seeds, so two builds given the same arguments analyse the same
+inputs and their --dump-outputs files can be compared array for array.
   value    : whole-job frames/s with the batch already resident in HBM (CUDA events around exactly K back-to-back passes, max over ranks)
   e2e      : the same metric through the public API `pylinac_b200.picketfence.analyze_batch` with HOST frames in page-locked memory --
              chunked H2D copies and the D2H of the results are inside the timed region; `e2e_pageable` is the same call on an
@@ -37,6 +40,7 @@ sys.path.insert(0, ROOT)
 FRAME_SHAPE = (1024, 1024)
 DPMM = 2.56
 PER_GPU_FRAMES = 512          # BASELINE.json configs[1]
+DUMP_LIMIT = 60_000_000      # array bytes written by --dump-outputs (with the .npy headers the files stay under 64 MB)
 METRIC = "EPID frames/sec (1024x1024) through PicketFence.analyze()"
 _SHARED_FRAMES = None         # frames handed to forked CPU workers
 
@@ -167,6 +171,24 @@ def _isolated(func, *args, chunked: bool = False):
             raise RuntimeError(f"{func.__name__} failed in the isolated process: {val}")
     proc.join()
     return result
+
+
+def dump_outputs(path, summary, meas):
+    """What analyze_batch returned in the last timed end-to-end step, one float64 array per field: summary_<field>.npy [n, ...] and
+    meas_<field>.npy [n, m, ...], where m is the largest measurement count of a frame (a frame's rows past its own count are zero),
+    and frame_index.npy, the batch index of every row.  A batch whose arrays exceed DUMP_LIMIT is written as a fixed seeded sample
+    of its frames."""
+    n, m = len(summary), int(summary["n_meas"].max())
+    width = lambda dt: sum(int(np.prod(dt[f].shape)) for f in dt.names)      # float64 values per row
+    per_frame = 8 * (1 + width(summary.dtype) + m * width(meas.dtype))
+    k = min(n, DUMP_LIMIT // per_frame)
+    idx = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "frame_index.npy"), idx.astype(np.float64))
+    for f in summary.dtype.names:
+        np.save(os.path.join(path, f"summary_{f}.npy"), summary[f][idx].astype(np.float64))
+    for f in meas.dtype.names:
+        np.save(os.path.join(path, f"meas_{f}.npy"), meas[f][idx, :m].astype(np.float64))
 
 
 def _gen_module_frames(kind_i):
@@ -376,7 +398,10 @@ def main():
     ap.add_argument("--frames", type=int, default=PER_GPU_FRAMES, help="frames per GPU per step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-modules", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed end-to-end step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -456,8 +481,8 @@ def main():
     barrier()
     clk = clocks.stop()
     assert all(int(s) == 0 for s in res.summary["status"]), "pipeline reported a failed frame"
-    # ---- the same call on pageable memory (fewer steps: it is slower)
-    psteps = max(2, min(args.steps, 5))
+    # ---- the same call on pageable memory
+    psteps = args.steps
     barrier()
     t0 = time.perf_counter()
     for _ in range(psteps):
@@ -579,7 +604,7 @@ def main():
                 mixed[i] = f
             mb = nat.Batch.upload(ctx, mixed)
             nat.pf_bench_timed(ctx, mb, params, 2)
-            msteps = max(3, min(args.steps, 10))
+            msteps = args.steps
             # every step of this workload has a host round trip (deferred count -> re-run): three repetitions, the fastest one is
             # reported (all three are listed: the spread is host scheduling, not the device)
             ex0 = ctx.counter(nat.CTR_PF_EXACT_FRAMES)
@@ -604,6 +629,8 @@ def main():
                 out["modules"] = bench_modules(ctx, nat, peak, cores)
             except Exception as e:  # pragma: no cover
                 out["modules"] = {"error": repr(e)}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res.summary, res.meas)
     print(json.dumps(out))
     if dist is not None:
         dist.barrier()

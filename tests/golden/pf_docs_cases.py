@@ -1,8 +1,8 @@
 """The reference's own PicketFence fixtures: the seven generated DICOM files under docs/source/files/ with the analyze() calls of
 their recipes (docs/source/picketfence.rst:455-730).  1280 x 1280, AS1200 pitch 0.336 mm, SID 1000.
 
-All seven FILES (header + pixel data, lzma-compressed, ~10 MB together) are committed in tests/golden/pf_docs_dcm.npz, so the GPU
-tests run every fixture on a box without /root/reference, and the file-level tests read them through pylinac_b200.dicom.
+All seven FILES (header + pixel data, lzma-compressed, ~10 MB together) are committed in tests/golden/pf_docs_dcm.npz; the GPU
+tests run every fixture from there, and the file-level tests read them through pylinac_b200.dicom.
 """
 from __future__ import annotations
 
@@ -11,7 +11,6 @@ import os
 
 import numpy as np
 
-REF_DIR = "/root/reference/docs/source/files"
 DCM_NPZ = os.path.join(os.path.dirname(__file__), "pf_docs_dcm.npz")
 PIXEL_MM, SHAPE = 0.336, (1280, 1280)
 # RTImageSID of each file (the docs recipes build three of them with AS1200Image(sid=1500), docs/source/picketfence.rst:551-667);
@@ -29,7 +28,6 @@ DOCS = {
     "offset_picket": {},
     "erroneous_leaves": {"separate_leaves": True, "nominal_gap_mm": 5},
 }
-COMMITTED = list(DOCS)
 
 
 def _pixel_tail(data: bytes):
@@ -38,20 +36,10 @@ def _pixel_tail(data: bytes):
     return np.frombuffer(data[-n:], dtype=np.uint16).reshape(SHAPE).copy()
 
 
-def available(name) -> bool:
-    return name in COMMITTED and os.path.exists(DCM_NPZ) or os.path.exists(os.path.join(REF_DIR, name + ".dcm"))
-
-
 def docs_dcm_bytes(name) -> bytes:
     """The complete DICOM file of a docs fixture."""
-    if name in COMMITTED and os.path.exists(DCM_NPZ):
-        with np.load(DCM_NPZ) as z:
-            return lzma.decompress(z[name].tobytes())
-    p = os.path.join(REF_DIR, name + ".dcm")
-    if os.path.exists(p):
-        with open(p, "rb") as f:
-            return f.read()
-    raise FileNotFoundError(name)
+    with np.load(DCM_NPZ) as z:
+        return lzma.decompress(z[name].tobytes())
 
 
 def docs_frame(name):

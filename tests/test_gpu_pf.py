@@ -89,8 +89,6 @@ def test_pf_matches_reference_on_docs_fixture(name):
     from pylinac_b200 import picketfence as pf
     from tests.golden import pf_docs_cases as dc
 
-    if not dc.available(name):
-        pytest.skip("frame not committed (noise makes it ~2 MB) and /root/reference is absent on this box")
     a, ps, sid, ak = dc.docs_frame(name)
     r = pf.analyze_batch(a[None], (1 / ps) * sid / 1000.0, **ak)[0]
     _compare_with_golden(r, name, np.load("tests/golden/pf_docs_golden.npz"))
@@ -306,9 +304,8 @@ def _leafband_cases():
             ck["mlc"] = pf.MLC.HD_MILLENNIUM
         out[nm] = (fr[None], (1 / ps) * sid / 1000.0, {**ck, **ak})
     for nm in ("rotated_up_down", "erroneous_leaves"):
-        if dc.available(nm):
-            fr, ps, sid, ak = dc.docs_frame(nm)
-            out["docs_" + nm] = (fr[None], (1 / ps) * sid / 1000.0, ak)
+        fr, ps, sid, ak = dc.docs_frame(nm)
+        out["docs_" + nm] = (fr[None], (1 / ps) * sid / 1000.0, ak)
     return out
 
 

@@ -66,13 +66,14 @@ def test_align_points_recovers_a_known_rigid_motion():
 def test_align_points_other_axes_orders_follow_the_reference_call():
     """winston_lutz.py:3592-3605, 3655-3658: any order of 'roll', 'pitch', 'yaw' is turned into an extrinsic euler string and the three
     angles of Rotation.as_euler are unpacked POSITIONALLY as (roll, pitch, yaw).  The default order also goes through scipy here and
-    must equal the closed form the module uses for it; the unmodified reference is called when it is importable."""
+    must equal the closed form the module uses for it; the unmodified reference's results are stored in tests/golden/fresh_golden.npz
+    (tests/golden/make_fresh_golden.py)."""
     from scipy.spatial.transform import Rotation
 
-    rng = np.random.default_rng(9)
-    pts = rng.uniform(-50, 50, size=(7, 3))
+    from tests.golden import fresh_cases as fc
+
+    pts, moved = fc.align_points_inputs()
     R = Rotation.from_euler("yxz", [2.2, -0.7, 1.5], degrees=True).as_matrix()
-    moved = pts @ R.T + np.array([0.4, -1.1, 2.0])
     mp_, ip_ = [Point(*q) for q in pts], [Point(*q) for q in moved]
     t0, y0, p0, r0 = mt.align_points(mp_, ip_)
     np.testing.assert_allclose([r0, p0, y0], [2.2, -0.7, 1.5], atol=1e-9)
@@ -85,14 +86,7 @@ def test_align_points_other_axes_orders_follow_the_reference_call():
         np.testing.assert_allclose(Rotation.from_euler(euler, [r, p, y], degrees=True).as_matrix(), R, atol=1e-12)
     with pytest.raises(KeyError):
         mt.align_points(mp_, ip_, axes_order="roll,pitch,spin")
-    try:
-        from oracle import refstub
-        ref = refstub.import_reference()
-        import pylinac.winston_lutz as rwl
-    except Exception:
-        return
-    RP = rwl.Point
-    for order in ("roll,pitch,yaw", "yaw,pitch,roll", "pitch,roll,yaw"):
-        tr, yr, pr, rr = rwl.align_points([RP(*q) for q in pts], [RP(*q) for q in moved], axes_order=order)
+    gold = np.load("tests/golden/fresh_golden.npz")
+    for order in fc.ALIGN_ORDERS:
         t, y, p, r = mt.align_points(mp_, ip_, axes_order=order)
-        np.testing.assert_allclose([y, p, r, t.x, t.y, t.z], [yr, pr, rr, tr.x, tr.y, tr.z], atol=1e-9, err_msg=order)
+        np.testing.assert_allclose([y, p, r, t.x, t.y, t.z], gold[f"align_points/{order}"], atol=1e-9, err_msg=order)

@@ -17,8 +17,6 @@ GOLD = np.load("tests/golden/pf_docs_golden.npz")
 
 @pytest.mark.parametrize("name", list(dc.DOCS))
 def test_oracle_matches_reference_on_docs_fixture(name):
-    if not dc.available(name):
-        pytest.skip("frame not committed and /root/reference is absent")
     a, ps, sid, ak = dc.docs_frame(name)
     sha = np.frombuffer(hashlib.sha1(a.tobytes()).digest(), dtype=np.uint8)
     assert np.array_equal(sha, GOLD[f"{name}/input_sha1"])

@@ -1,24 +1,15 @@
-"""The restated image generator (oracle/synth.py, test infrastructure) against the pieces of the reference's generator that run here
-without scikit-image: the BB projection of generate_winstonlutz (winston_lutz.py:3401-3460)."""
-import os
-
+"""The restated image generator (oracle/synth.py, test infrastructure) against the pieces of the reference's generator that run
+without scikit-image: the BB projection of generate_winstonlutz (winston_lutz.py:3401-3460), whose outputs on 300 random setups are
+stored in tests/golden/fresh_golden.npz (tests/golden/make_fresh_golden.py)."""
 import numpy as np
-import pytest
 
 from oracle import synth
-
-pytestmark = pytest.mark.skipif(not os.path.isdir("/root/reference/pylinac"), reason="needs the reference tree")
+from tests.golden import fresh_cases as fc
 
 
 def test_bb_projection_matches_the_reference_function():
-    from oracle.refstub import import_reference
-
-    import_reference()
-    from pylinac.winston_lutz import bb_projection_with_rotation as ref
-
-    rng = np.random.default_rng(0)
-    for _ in range(300):
-        left, up, inn = rng.uniform(-5, 5, 3)
-        g, c = rng.uniform(0, 360, 2)
-        a, b = ref(left, up, inn, g, c), synth.bb_projection_with_rotation(left, up, inn, g, c)
-        assert abs(a[0] - b[0]) < 1e-12 and abs(a[1] - b[1]) < 1e-12
+    gold = np.load("tests/golden/fresh_golden.npz")
+    x = gold["bb_projection/inputs"]
+    np.testing.assert_array_equal(x, fc.bb_projection_inputs())
+    ours = np.array([synth.bb_projection_with_rotation(*row) for row in x])
+    assert np.max(np.abs(ours - gold["bb_projection/outputs"])) < 1e-12
