@@ -54,13 +54,11 @@ int32_t epid_version(void);
 /* options / diagnostic counters (no reference counterpart: the reference has a single CPU code path).
  * EPID_OPT_PF_EXACT_ONLY: 1 = always use the exact-histogram PicketFence pipeline (default 0: fused sample-guided front
  * kernel with automatic per-batch fallback to the exact pipeline).  EPID_CTR_PF_FALLBACKS: batches / chunks re-run exactly. */
-enum { EPID_OPT_PF_EXACT_ONLY = 1, EPID_OPT_PF_LEAFBAND = 2 /* 1 = experimental leaf-band window kernel (bit-identical results; default 0) */,
+/* Keys 2, 4 and 6 are retired and not reused: epid_set_option rejects them as unknown. */
+enum { EPID_OPT_PF_EXACT_ONLY = 1,
        EPID_OPT_PF_WIN2 = 3 /* 1 (default) = two-kernel window path (medians + per-window analysis); 0 = single per-window kernel (bit-identical) */,
-       EPID_OPT_PF_SPLIT = 4 /* S >= 2: a device-resident batch runs as S sub-batches on S streams, so that the latency-bound per-frame
-                                kernels of one sub-batch overlap the streaming kernels of another (bit-identical results); 0 / 1 = one stream */,
        EPID_OPT_PF_FAST_REDO = 5 /* 1 (default): a deferred frame whose _has_noise() == True can be certified by one exact count is median-filtered
                                     and re-run by the certified fast pipeline; 0 = every deferred frame goes to the exact-histogram pipeline */,
-       EPID_OPT_PF_OVERLAP_REDO = 6 /* 1 (default): epid_pf_analyze re-runs deferred frames on a second stream while the batch's window stages run */,
        EPID_OPT_STATS_EXACT = 7 /* 1: FieldAnalysis / Starshot compute check_inversion_by_histogram from the exact histogram for every frame
                                    (default 0: decision certified from exact counts at pilot thresholds, exact histogram only where that fails) */ };
 enum { EPID_CTR_PF_FALLBACKS = 1, EPID_CTR_PF_REDONE_FRAMES = 2 /* frames re-run individually (fast re-run or exact pipeline) */,
@@ -248,15 +246,12 @@ int32_t epid_pf_analyze_host(epid_ctx* ctx, const uint16_t* frames, int32_t n, i
 int32_t epid_pf_bench(epid_ctx* ctx, const epid_batch* frames, const epid_pf_params* p, int32_t iters,
                       float* total_ms, float* stats_kernel_ms, int64_t* launches);
 /* the same timed region with CUDA-event marks between the kernels: total_ms of `iters` back-to-back passes, stage_ms[k] summed over
- * the passes (stage ids as for epid_pf_bench_stages), kernel launches and the number of frames the per-frame exact fallback re-ran
- * (when the batch contains deferred frames the passes are timed with the host round trip of the fallback included) */
+ * the passes, kernel launches and the number of frames the per-frame exact fallback re-ran (when the batch contains deferred frames
+ * the passes are timed with the host round trip of the fallback included).  stage_ms[0..8] (bench.py's per-kernel roofline table) =
+ * init + pilot, stream, tail, windows (per-window kernel), windows (generic), finalize, exact front end (fallback only), windows
+ * (two-kernel path: medians), windows (two-kernel path: per-window analysis) */
 int32_t epid_pf_bench_timed(epid_ctx* ctx, const epid_batch* frames, const epid_pf_params* p, int32_t iters, float* total_ms,
                             float* stage_ms, int32_t nstages, int64_t* launches, int64_t* redone_frames);
-/* per-stage device times of `iters` passes (CUDA events between the kernels; bench.py's per-kernel roofline table):
- * stage_ms[0..9] = init + pilot, stream, tail, windows (per-window kernel), windows (generic), finalize, exact front end (fallback
- * only), windows (leaf-band kernel), windows (two-kernel path: medians), windows (two-kernel path: per-window analysis) */
-int32_t epid_pf_bench_stages(epid_ctx* ctx, const epid_batch* frames, const epid_pf_params* p, int32_t iters, float* stage_ms,
-                             int32_t nstages);
 
 
 /* ----------------------------------------------------------------------------------------- Starshot

@@ -24,11 +24,8 @@ _NP2DT = {np.dtype(np.uint8): U8, np.dtype(np.uint16): U16, np.dtype(np.int32): 
 _DT2NP = {v: k for k, v in _NP2DT.items()}
 
 OPT_PF_EXACT_ONLY = 1
-OPT_PF_LEAFBAND = 2
 OPT_PF_WIN2 = 3
-OPT_PF_SPLIT = 4
 OPT_PF_FAST_REDO = 5
-OPT_PF_OVERLAP_REDO = 6
 OPT_STATS_EXACT = 7
 CTR_PF_FALLBACKS = 1
 CTR_PF_REDONE_FRAMES = 2
@@ -301,7 +298,6 @@ _SIGNATURES = {
     "epid_pf_analyze_host": [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.POINTER(PFParams), _P, _P, C.c_int32],
     "epid_pf_bench": [_P, _P, C.POINTER(PFParams), C.c_int32, C.POINTER(C.c_float), C.POINTER(C.c_float),
                       C.POINTER(C.c_int64)],
-    "epid_pf_bench_stages": [_P, _P, C.POINTER(PFParams), C.c_int32, C.POINTER(C.c_float), C.c_int32],
     "epid_pf_bench_timed": [_P, _P, C.POINTER(PFParams), C.c_int32, C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_int32,
                             C.POINTER(C.c_int64), C.POINTER(C.c_int64)],
     "epid_starshot_analyze": [_P, _P, C.POINTER(StarParams), _P, _P, C.c_int32, _P],
@@ -633,7 +629,7 @@ def pf_bench(ctx: Context, batch: Batch, params: PFParams, iters: int):
 
 
 PF_STAGE_NAMES = ("k_pf_init + k_pf_pilot", "k_pf_stream", "k_pf_tail", "k_pf_windows_fast", "k_pf_windows (generic)", "k_pf_finalize",
-                  "exact front end (fallback)", "k_pf_leafband", "k_pf_win_medians", "k_pf_win_fwxm")
+                  "exact front end (fallback)", "k_pf_win_medians", "k_pf_win_fwxm")
 
 
 def pf_bench_timed(ctx: Context, batch: Batch, params: PFParams, iters: int):
@@ -648,9 +644,7 @@ def pf_bench_timed(ctx: Context, batch: Batch, params: PFParams, iters: int):
 
 def pf_bench_stages(ctx: Context, batch: Batch, params: PFParams, iters: int) -> dict:
     """{stage name: ms per pass} from CUDA events recorded between the kernels of `iters` device-resident passes."""
-    out = (C.c_float * 16)()
-    check(lib().epid_pf_bench_stages(ctx.handle, batch.handle, C.byref(params), iters, out, 16))
-    return {name: out[k] / iters for k, name in enumerate(PF_STAGE_NAMES)}
+    return pf_bench_timed(ctx, batch, params, iters)[1]
 
 
 def gaussian_kernel_table(max_sigma: int):

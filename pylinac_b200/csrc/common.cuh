@@ -70,15 +70,11 @@ struct epid_ctx {
     size_t pinned_ring_bytes = 0;
     // options / diagnostics (epid_set_option / epid_get_counter)
     int pf_exact_only = 0;               // 1: never use the fused sample-guided front kernel
-    int pf_leafband = 0;                 // 1: experimental leaf-band window kernel for the frames it covers (default: per-window kernel)
-    int pf_split = 0;                    // >= 2: sub-batches on that many streams (EPID_OPT_PF_SPLIT)
-    cudaStream_t aux_stream[4] = {nullptr, nullptr, nullptr, nullptr};   // created on first use
     int pf_win2 = 1;                     // 1 (default): two-kernel window path for the frames it covers (pf_windows2.cu)
     int64_t pf_fallbacks = 0;            // batches (or chunks) re-run by the exact pipeline
     int64_t pf_redone_frames = 0;        // frames re-run individually (per-frame fallback: certified-noise fast re-run or exact pipeline)
     int64_t pf_exact_frames = 0;         // of those, frames that needed the exact-histogram pipeline
     int pf_fast_redo = 1;                // 1 (default): deferred frames whose noise flag can be certified are median-filtered and re-run by the fast pipeline
-    int pf_overlap_redo = 1;             // 1 (default): device-resident batches re-run their deferred frames on redo_stream while the batch's window stages run
     cudaStream_t redo_stream = nullptr;  // high-priority stream of the per-frame re-run
     cudaEvent_t ev_front = nullptr, ev_main_done = nullptr, ev_redo_done = nullptr;
     int* h_flags = nullptr;              // 64 page-locked, device-mapped ints: [0] deferred count written by k_pf_collect_deferred

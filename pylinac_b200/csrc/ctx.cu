@@ -120,7 +120,6 @@ int32_t epid_ctx_destroy(epid_ctx* ctx) {
     if (ctx->pinned_ring) cudaFreeHost(ctx->pinned_ring);
     if (ctx->pinned) cudaFreeHost(ctx->pinned);
     cudaStreamDestroy(ctx->stream);
-    for (int k = 0; k < 4; k++) if (ctx->aux_stream[k]) cudaStreamDestroy(ctx->aux_stream[k]);
     cudaStreamDestroy(ctx->copy_stream[0]);
     cudaStreamDestroy(ctx->copy_stream[1]);
     if (ctx->redo_stream) { cudaStreamSynchronize(ctx->redo_stream); cudaStreamDestroy(ctx->redo_stream); }
@@ -164,11 +163,8 @@ int32_t epid_set_option(epid_ctx* ctx, int32_t key, int64_t value) {
     EPID_REQUIRE(ctx, EPID_ERR_INVALID, "ctx is NULL");
     switch (key) {
         case EPID_OPT_PF_EXACT_ONLY: ctx->pf_exact_only = value ? 1 : 0; return EPID_OK;
-        case EPID_OPT_PF_LEAFBAND: ctx->pf_leafband = value ? 1 : 0; return EPID_OK;
         case EPID_OPT_PF_WIN2: ctx->pf_win2 = value ? 1 : 0; return EPID_OK;
-        case EPID_OPT_PF_SPLIT: ctx->pf_split = value < 2 ? 0 : (value > 4 ? 4 : (int)value); return EPID_OK;
         case EPID_OPT_PF_FAST_REDO: ctx->pf_fast_redo = value ? 1 : 0; return EPID_OK;
-        case EPID_OPT_PF_OVERLAP_REDO: ctx->pf_overlap_redo = value ? 1 : 0; return EPID_OK;
         case EPID_OPT_STATS_EXACT: ctx->stats_exact = value ? 1 : 0; return EPID_OK;
     }
     set_error("unknown option %d", key);

@@ -377,7 +377,7 @@ int32_t epid_frame_stats(epid_ctx* ctx, const epid_batch* b, int32_t r0, int32_t
     uint32_t* d_col = (uint32_t*)p;
     k_refs_from_batch<<<(n + 127) / 128, 128, 0, ctx->stream>>>(base, n, b->h, b->w, r0, c0, refs);
     ctx->launches++;
-    rc = launch_frame_stats(ctx, ctx->stream, g, refs, nullptr, n, st, d_row, d_col);
+    rc = launch_frame_stats(ctx, ctx->stream, g, refs, n, st, d_row, d_col);
     std::vector<FrameStats> hs(n);
     std::vector<uint32_t> hrow, hcol;
     if (rc == EPID_OK) {

@@ -616,8 +616,7 @@ static int pf_run(epid_ctx* ctx, cudaStream_t stream, const uint16_t* d_frames, 
     hc.W = W;
     hc.meas_cap = meas_cap;
     hc.post_filter = 0;
-    hc.leafband = ctx->pf_leafband ? 1 : 0;
-    hc.win2 = (ctx->pf_win2 && !hc.leafband) ? 1 : 0;
+    hc.win2 = ctx->pf_win2;
     const int npix = H * W;
     hc.lo = pct_plan(npix, 0.5);
     hc.hi = pct_plan(npix, 99.5);
@@ -658,7 +657,7 @@ static int pf_run(epid_ctx* ctx, cudaStream_t stream, const uint16_t* d_frames, 
         if (front_evt) EPID_CUDA(cudaEventRecord(front_evt, stream));
     } else {
         if (tm && tm->on) { rc = tm->record(stream); if (rc != EPID_OK) return rc; }
-        rc = launch_frame_stats(ctx, stream, g, w.refs, nullptr, n, w.stats, w.rowsum, w.colsum);
+        rc = launch_frame_stats(ctx, stream, g, w.refs, n, w.stats, w.rowsum, w.colsum);
         if (rc == EPID_OK && tm && tm->on) rc = tm->record(stream);
     }
     if (rc != EPID_OK) return rc;
@@ -696,7 +695,7 @@ static int pf_run(epid_ctx* ctx, cudaStream_t stream, const uint16_t* d_frames, 
         // would recompute identical numbers, so run it on all frames -- flagged ones are rare and this keeps
         // one code path.
         EPID_CUDA(cudaMemsetAsync(w.counters, 0, sizeof(int), stream));
-        rc = launch_frame_stats(ctx, stream, g, w.refs, nullptr, n, w.stats, w.rowsum, w.colsum);
+        rc = launch_frame_stats(ctx, stream, g, w.refs, n, w.stats, w.rowsum, w.colsum);
         if (rc != EPID_OK) return rc;
         k_pf_decide<<<nb, tb, 0, stream>>>(w.cst, w.stats, w.fr, n, w.select, 1, w.counters);
         ctx->launches++;
@@ -720,7 +719,7 @@ static int pf_run(epid_ctx* ctx, cudaStream_t stream, const uint16_t* d_frames, 
         EPID_CUDA(cudaMemcpyAsync(w.cst, &hc, sizeof(hc), cudaMemcpyHostToDevice, stream));
         StatsGeom g2 = g;
         g2.box = 0;
-        rc = launch_frame_stats(ctx, stream, g2, w.refs, nullptr, n, w.stats, w.rowsum, w.colsum);
+        rc = launch_frame_stats(ctx, stream, g2, w.refs, n, w.stats, w.rowsum, w.colsum);
         if (rc != EPID_OK) return rc;
         k_pf_decide<<<nb, tb, 0, stream>>>(w.cst, w.stats, w.fr, n, nullptr, 0, w.counters);
         ctx->launches++;
@@ -743,11 +742,6 @@ static int pf_run(epid_ctx* ctx, cudaStream_t stream, const uint16_t* d_frames, 
     }   // !fast
     {
         // fast path for ordinary window sizes, then the generic kernel for whatever it left marked (valid == -1)
-        if (hc.leafband) {
-            rc = launch_pf_leafband(ctx, stream, w.cst, w.refs, w.fr, w.wins, n);
-            if (rc != EPID_OK) return rc;
-            if (tm) { rc = tm->mark(stream, PF_STAGE_LEAFBAND); if (rc != EPID_OK) return rc; }
-        }
         if (hc.win2) {
             rc = launch_pf_windows2(ctx, stream, w.cst, w.refs, w.fr, w.winrec, w.wins, n, tm);
             if (rc != EPID_OK) return rc;
@@ -988,55 +982,6 @@ struct PfResultCopy {   // async D2H of one chunk's results + the counters ([2] 
 
 }  // namespace
 
-// S sub-batches on S streams (EPID_OPT_PF_SPLIT): every sub-batch is a complete, independent pipeline with its own work area, so the
-// results are those of the single-stream run; the streams fork from and join into ctx->stream.
-struct PfSplit {
-    int S = 0;
-    PfWork w[4];
-    int n0[4], nn[4];
-    cudaStream_t st[4];
-    cudaEvent_t fork = nullptr, join[4] = {nullptr, nullptr, nullptr, nullptr};
-    int prepare(epid_ctx* ctx, int n, int H, int W, int meas_cap) {
-        S = ctx->pf_split < n ? ctx->pf_split : n;
-        if (S < 2) { S = 0; return EPID_OK; }
-        size_t tot = 0, off[4];
-        for (int k = 0; k < S; k++) {
-            n0[k] = (int)((long long)n * k / S);
-            nn[k] = (int)((long long)n * (k + 1) / S) - n0[k];
-            carve(w[k], nullptr, nn[k], H, W, meas_cap);
-            off[k] = tot;
-            tot += align_up(w[k].total, 512);
-        }
-        int rc = ensure_scratch(ctx, tot);
-        if (rc != EPID_OK) return rc;
-        for (int k = 0; k < S; k++) carve(w[k], (char*)ctx->scratch + off[k], nn[k], H, W, meas_cap);
-        st[0] = ctx->stream;
-        for (int k = 1; k < S; k++) {
-            if (!ctx->aux_stream[k]) EPID_CUDA(cudaStreamCreateWithFlags(&ctx->aux_stream[k], cudaStreamNonBlocking));
-            st[k] = ctx->aux_stream[k];
-        }
-        EPID_CUDA(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
-        for (int k = 1; k < S; k++) EPID_CUDA(cudaEventCreateWithFlags(&join[k], cudaEventDisableTiming));
-        return EPID_OK;
-    }
-    int do_fork(epid_ctx* ctx) {
-        EPID_CUDA(cudaEventRecord(fork, ctx->stream));
-        for (int k = 1; k < S; k++) EPID_CUDA(cudaStreamWaitEvent(st[k], fork, 0));
-        return EPID_OK;
-    }
-    int do_join(epid_ctx* ctx) {
-        for (int k = 1; k < S; k++) {
-            EPID_CUDA(cudaEventRecord(join[k], st[k]));
-            EPID_CUDA(cudaStreamWaitEvent(ctx->stream, join[k], 0));
-        }
-        return EPID_OK;
-    }
-    void destroy() {
-        if (fork) cudaEventDestroy(fork);
-        for (int k = 1; k < 4; k++) if (join[k]) cudaEventDestroy(join[k]);
-    }
-};
-
 extern "C" {
 
 int32_t epid_pf_analyze(epid_ctx* ctx, const epid_batch* frames, const epid_pf_params* p, epid_pf_summary* summary,
@@ -1054,61 +999,16 @@ int32_t epid_pf_analyze(epid_ctx* ctx, const epid_batch* frames, const epid_pf_p
     carve(w, (char*)ctx->scratch, n, H, W, meas_cap);
     uint16_t* pools[3] = {nullptr, nullptr, nullptr};
     const bool fast = pf_fast_ok(ctx, p, frames->h, frames->w);
-    auto copy_and_wait = [&](int* cnt3) -> int {
-        int r = PfResultCopy::enqueue(ctx->stream, w, n, meas_cap, summary, meas, cnt3);
-        cudaError_t e = cudaStreamSynchronize(ctx->stream);
-        if (r == EPID_OK && e != cudaSuccess) { set_error("PF pipeline failed: %s", cudaGetErrorString(e)); r = EPID_ERR_CUDA; }
-        return r;
-    };
+    // the re-run of deferred frames (if any) overlaps the window stages of the batch on ctx->redo_stream; the exact pipeline defers none
+    int m = 0;
+    const uint16_t* d_frames = (const uint16_t*)frames->dptr;
+    rc = fast ? pf_run_overlapped(ctx, ctx->stream, d_frames, n, frames->h, frames->w, p, meas_cap, w, pools, nullptr, &m)
+              : pf_run(ctx, ctx->stream, d_frames, n, frames->h, frames->w, p, meas_cap, w, pools, nullptr, false);
+    if (m > 0) ctx->pf_fallbacks++;
     int cnt3[3] = {0, 0, 0};
-    if (fast && ctx->pf_split >= 2 && n >= 2 * ctx->pf_split) {
-        // sub-batches on several streams, each with its own work area; result rows are copied per sub-batch.  A sub-batch with
-        // deferred frames makes the call fall back to the single-stream path below (rare: noisy / undecidable frames).
-        PfSplit sp;
-        rc = sp.prepare(ctx, n, H, W, meas_cap);
-        bool deferred = false;
-        if (rc == EPID_OK && sp.S >= 2) {
-            const size_t per = (size_t)frames->h * frames->w;
-            rc = sp.do_fork(ctx);
-            int cnt[4][3] = {};
-            for (int k = 0; k < sp.S && rc == EPID_OK; k++) {
-                rc = pf_run(ctx, sp.st[k], (const uint16_t*)frames->dptr + per * sp.n0[k], sp.nn[k], frames->h, frames->w, p, meas_cap, sp.w[k],
-                            pools, nullptr, true);
-                if (rc == EPID_OK) rc = PfResultCopy::enqueue(sp.st[k], sp.w[k], sp.nn[k], meas_cap, summary + sp.n0[k], meas + (size_t)sp.n0[k] * meas_cap, cnt[k]);
-            }
-            if (rc == EPID_OK) rc = sp.do_join(ctx);
-            cudaError_t e = cudaStreamSynchronize(ctx->stream);
-            for (int k = 1; k < sp.S; k++) cudaStreamSynchronize(sp.st[k]);
-            if (rc == EPID_OK && e != cudaSuccess) { set_error("PF pipeline failed: %s", cudaGetErrorString(e)); rc = EPID_ERR_CUDA; }
-            for (int k = 0; k < sp.S; k++) deferred = deferred || cnt[k][2] > 0;
-        }
-        sp.destroy();
-        if (rc != EPID_OK || (sp.S >= 2 && !deferred)) {
-            for (int k = 0; k < 3; k++) if (pools[k]) cudaFree(pools[k]);
-            return rc;
-        }
-        rc = ensure_scratch(ctx, w.total);
-        if (rc != EPID_OK) return rc;
-        carve(w, (char*)ctx->scratch, n, H, W, meas_cap);
-    }
-    if (fast && ctx->pf_overlap_redo) {
-        // the re-run of deferred frames (if any) overlaps the window stages of the batch on ctx->redo_stream
-        int m = 0;
-        rc = pf_run_overlapped(ctx, ctx->stream, (const uint16_t*)frames->dptr, n, frames->h, frames->w, p, meas_cap, w, pools, nullptr, &m);
-        if (m > 0) ctx->pf_fallbacks++;
-        if (rc == EPID_OK) rc = copy_and_wait(cnt3); else cudaStreamSynchronize(ctx->stream);
-        for (int k = 0; k < 3; k++) if (pools[k]) cudaFree(pools[k]);
-        return rc;
-    }
-    rc = pf_run(ctx, ctx->stream, (const uint16_t*)frames->dptr, n, frames->h, frames->w, p, meas_cap, w, pools, nullptr, fast);
-    if (rc == EPID_OK) rc = copy_and_wait(cnt3); else cudaStreamSynchronize(ctx->stream);
-    if (rc == EPID_OK && fast && cnt3[2] > 0) {
-        // frames the certified front end deferred (noise candidates, undecidable orientation): exactly those are re-run
-        ctx->pf_fallbacks++;
-        int dummy[3];
-        rc = pf_redo_deferred(ctx, ctx->stream, (const uint16_t*)frames->dptr, cnt3[2], frames->h, frames->w, p, meas_cap, w, pools);
-        if (rc == EPID_OK) rc = copy_and_wait(dummy); else cudaStreamSynchronize(ctx->stream);
-    }
+    if (rc == EPID_OK) rc = PfResultCopy::enqueue(ctx->stream, w, n, meas_cap, summary, meas, cnt3);
+    cudaError_t e = cudaStreamSynchronize(ctx->stream);
+    if (rc == EPID_OK && e != cudaSuccess) { set_error("PF pipeline failed: %s", cudaGetErrorString(e)); rc = EPID_ERR_CUDA; }
     for (int k = 0; k < 3; k++) if (pools[k]) cudaFree(pools[k]);
     return rc;
 }
@@ -1130,51 +1030,13 @@ static int32_t pf_bench_impl(epid_ctx* ctx, const epid_batch* frames, const epid
     carve(w, (char*)ctx->scratch, n, H, W, meas_cap);
     uint16_t* pools[3] = {nullptr, nullptr, nullptr};
     const bool fast = pf_fast_ok(ctx, p, frames->h, frames->w);
+    const uint16_t* d_frames = (const uint16_t*)frames->dptr;
     cudaEvent_t t0, t1;
     EPID_CUDA(cudaEventCreate(&t0));
     EPID_CUDA(cudaEventCreate(&t1));
-    if (fast && ctx->pf_split >= 2 && n >= 2 * ctx->pf_split && !stage_ms) {
-        // sub-batches on several streams; falls through to the single-stream path when a frame was deferred
-        PfSplit sp;
-        rc = sp.prepare(ctx, n, H, W, meas_cap);
-        bool deferred = false;
-        if (rc == EPID_OK && sp.S >= 2) {
-            const int64_t l0 = ctx->launches;
-            const size_t per = (size_t)frames->h * frames->w;
-            EPID_CUDA(cudaStreamSynchronize(ctx->stream));
-            EPID_CUDA(cudaEventRecord(t0, ctx->stream));
-            rc = sp.do_fork(ctx);
-            for (int it = 0; it < iters && rc == EPID_OK; it++)
-                for (int k = 0; k < sp.S && rc == EPID_OK; k++)
-                    rc = pf_run(ctx, sp.st[k], (const uint16_t*)frames->dptr + per * sp.n0[k], sp.nn[k], frames->h, frames->w, p, meas_cap, sp.w[k],
-                                pools, nullptr, true);
-            if (rc == EPID_OK) rc = sp.do_join(ctx);
-            cudaEventRecord(t1, ctx->stream);
-            int cnt[4][3] = {};
-            for (int k = 0; k < sp.S; k++) cudaMemcpyAsync(cnt[k], sp.w[k].counters, sizeof(cnt[k]), cudaMemcpyDeviceToHost, ctx->stream);
-            cudaStreamSynchronize(ctx->stream);
-            for (int k = 1; k < sp.S; k++) cudaStreamSynchronize(sp.st[k]);
-            for (int k = 0; k < sp.S; k++) deferred = deferred || cnt[k][2] > 0;
-            float ms = 0;
-            cudaEventElapsedTime(&ms, t0, t1);
-            if (total_ms) *total_ms = ms;
-            if (stats_kernel_ms) *stats_kernel_ms = 0.f;
-            if (launches) *launches = ctx->launches - l0;
-            if (redone) *redone = 0;
-        }
-        sp.destroy();
-        if (rc != EPID_OK || (sp.S >= 2 && !deferred)) {
-            cudaEventDestroy(t0); cudaEventDestroy(t1);
-            for (int k = 0; k < 3; k++) if (pools[k]) cudaFree(pools[k]);
-            return rc;
-        }
-        // carve() above re-used the scratch: restore the single-batch work area
-        rc = ensure_scratch(ctx, w.total);
-        if (rc != EPID_OK) return rc;
-        carve(w, (char*)ctx->scratch, n, H, W, meas_cap);
-    }
     // pass 0: back-to-back passes, no host round trip (what an ordinary batch costs).  If that left deferred frames, pass 1 times
-    // the real control flow: after every fast pass the host reads the deferred count and enqueues the per-frame exact re-run.
+    // the real control flow of epid_pf_analyze: after the front end of every pass the host reads the deferred count and runs the
+    // per-frame re-run on ctx->redo_stream, overlapped with the batch's window stages.
     for (int mode = 0; mode < 2; mode++) {
         PfTimers tm;
         tm.on = true;
@@ -1183,18 +1045,9 @@ static int32_t pf_bench_impl(epid_ctx* ctx, const epid_batch* frames, const epid
         int cnt3[3] = {0, 0, 0};
         EPID_CUDA(cudaStreamSynchronize(ctx->stream));
         EPID_CUDA(cudaEventRecord(t0, ctx->stream));
-        for (int it = 0; it < iters && rc == EPID_OK; it++) {
-            if (mode == 1 && ctx->pf_overlap_redo) {
-                rc = pf_run_overlapped(ctx, ctx->stream, (const uint16_t*)frames->dptr, n, frames->h, frames->w, p, meas_cap, w, pools, &tm, nullptr);
-                continue;
-            }
-            rc = pf_run(ctx, ctx->stream, (const uint16_t*)frames->dptr, n, frames->h, frames->w, p, meas_cap, w, pools, &tm, fast);
-            if (mode == 1 && rc == EPID_OK) {
-                cudaMemcpyAsync(cnt3, w.counters, sizeof(cnt3), cudaMemcpyDeviceToHost, ctx->stream);
-                cudaStreamSynchronize(ctx->stream);
-                if (cnt3[2] > 0) rc = pf_redo_deferred(ctx, ctx->stream, (const uint16_t*)frames->dptr, cnt3[2], frames->h, frames->w, p, meas_cap, w, pools);
-            }
-        }
+        for (int it = 0; it < iters && rc == EPID_OK; it++)
+            rc = mode == 0 ? pf_run(ctx, ctx->stream, d_frames, n, frames->h, frames->w, p, meas_cap, w, pools, &tm, fast)
+                           : pf_run_overlapped(ctx, ctx->stream, d_frames, n, frames->h, frames->w, p, meas_cap, w, pools, &tm, nullptr);
         cudaEventRecord(t1, ctx->stream);
         if (mode == 0) cudaMemcpyAsync(cnt3, w.counters, sizeof(cnt3), cudaMemcpyDeviceToHost, ctx->stream);
         cudaStreamSynchronize(ctx->stream);
@@ -1222,34 +1075,6 @@ int32_t epid_pf_bench(epid_ctx* ctx, const epid_batch* frames, const epid_pf_par
 int32_t epid_pf_bench_timed(epid_ctx* ctx, const epid_batch* frames, const epid_pf_params* p, int32_t iters, float* total_ms, float* stage_ms,
                             int32_t nstages, int64_t* launches, int64_t* redone_frames) {
     return pf_bench_impl(ctx, frames, p, iters, total_ms, nullptr, launches, stage_ms, nstages, redone_frames);
-}
-
-int32_t epid_pf_bench_stages(epid_ctx* ctx, const epid_batch* frames, const epid_pf_params* p, int32_t iters, float* stage_ms, int32_t nstages) {
-    EPID_REQUIRE(ctx && frames && p && stage_ms && iters > 0 && nstages >= PF_NSTAGES, EPID_ERR_INVALID, "bad argument");
-    EPID_REQUIRE(frames->dtype == EPID_U16, EPID_ERR_UNSUPPORTED, "picket fence frames must be uint16");
-    const int meas_cap = 1024;
-    int rc = pf_validate(p, frames->h, frames->w, meas_cap);
-    if (rc != EPID_OK) return rc;
-    EPID_CUDA(cudaSetDevice(ctx->device));
-    const int n = frames->n, H = frames->h - 2 * p->crop_px, W = frames->w - 2 * p->crop_px;
-    PfWork w;
-    carve(w, nullptr, n, H, W, meas_cap);
-    rc = ensure_scratch(ctx, w.total);
-    if (rc != EPID_OK) return rc;
-    carve(w, (char*)ctx->scratch, n, H, W, meas_cap);
-    uint16_t* pools[3] = {nullptr, nullptr, nullptr};
-    const bool fast = pf_fast_ok(ctx, p, frames->h, frames->w);
-    PfTimers tm;
-    tm.stages = true;
-    EPID_CUDA(cudaStreamSynchronize(ctx->stream));
-    for (int it = 0; it < iters && rc == EPID_OK; it++)
-        rc = pf_run(ctx, ctx->stream, (const uint16_t*)frames->dptr, n, frames->h, frames->w, p, meas_cap, w, pools, &tm, fast);
-    cudaError_t e = cudaStreamSynchronize(ctx->stream);
-    if (rc == EPID_OK && e != cudaSuccess) { set_error("PF pipeline failed: %s", cudaGetErrorString(e)); rc = EPID_ERR_CUDA; }
-    if (rc == EPID_OK) tm.stage_ms(stage_ms, PF_NSTAGES);
-    tm.destroy();
-    for (int k = 0; k < 3; k++) if (pools[k]) cudaFree(pools[k]);
-    return rc;
 }
 
 int32_t epid_pf_analyze_host(epid_ctx* ctx, const uint16_t* frames, int32_t n, int32_t h, int32_t w_, const epid_pf_params* p,
@@ -1343,7 +1168,7 @@ int32_t epid_pf_analyze_host(epid_ctx* ctx, const uint16_t* frames, int32_t n, i
         if (fast && h_cnt[s][2] > 0) {     // re-run exactly the frames the front end deferred, then fetch the chunk's rows again
             ctx->pf_fallbacks++;
             // on the re-run stream: the chunk's own pass has finished, the next chunk's pass keeps ctx->stream busy meanwhile
-            cudaStream_t rs = ctx->pf_overlap_redo ? ctx->redo_stream : ctx->stream;
+            cudaStream_t rs = ctx->redo_stream;
             int r = pf_redo_deferred(ctx, rs, bufs[s], h_cnt[s][2], h, w_, p, meas_cap, works[s], pools);
             if (r != EPID_OK) return r;
             r = PfResultCopy::enqueue(rs, works[s], cnt, meas_cap, direct ? summary + (size_t)ci * chunk : h_summ[s],

@@ -30,7 +30,6 @@ struct PfConst {
     int H, W;
     int meas_cap;
     int post_filter;       // stats were taken on an already inverted+filtered copy
-    int leafband;          // 1: frames the leaf-band window kernel covers are processed by it (pf_windows.cu)
     int win2;              // 1: frames the two-kernel window path covers are processed by it (pf_windows2.cu)
     PctPlan lo, hi;        // p0.5 / p99.5 of the frame (ranks live in StatsGeom slots 0..3)
     PctPlan p85[2], p99[2];  // [0]: arrays of length W (np.sum(axis 0)), [1]: length H
@@ -127,7 +126,7 @@ struct PfTimers {
         for (size_t i = 0; i + 1 < ev.size(); i += 2) { float ms = 0; cudaEventElapsedTime(&ms, ev[i], ev[i + 1]); t += ms; }
         return t;
     }
-    // stage marks (epid_pf_bench_stages): the time between two consecutive marks is charged to the later mark's stage id
+    // stage marks (epid_pf_bench_timed): the time between two consecutive marks is charged to the later mark's stage id
     bool stages = false;
     std::vector<std::pair<int, cudaEvent_t>> marks;
     int mark(cudaStream_t s, int stage) {
@@ -156,11 +155,10 @@ struct PfTimers {
     }
 };
 enum { PF_STAGE_START = -1, PF_STAGE_INIT_PILOT = 0, PF_STAGE_STREAM = 1, PF_STAGE_TAIL = 2, PF_STAGE_WINDOWS = 3, PF_STAGE_WINDOWS_GENERIC = 4,
-       PF_STAGE_FINALIZE = 5, PF_STAGE_EXACT_FRONT = 6, PF_STAGE_LEAFBAND = 7, PF_STAGE_WIN_MEDIANS = 8, PF_STAGE_WIN_FWXM = 9, PF_NSTAGES = 10 };
+       PF_STAGE_FINALIZE = 5, PF_STAGE_EXACT_FRONT = 6, PF_STAGE_WIN_MEDIANS = 7, PF_STAGE_WIN_FWXM = 8, PF_NSTAGES = 9 };
 
 // pf_windows.cu
 int launch_pf_windows_fast(epid_ctx* ctx, cudaStream_t stream, const PfConst* cst, const FrameRef* refs, PfFrame* fr, PfWin* wins, int n);
-int launch_pf_leafband(epid_ctx* ctx, cudaStream_t stream, const PfConst* cst, const FrameRef* refs, PfFrame* fr, PfWin* wins, int n);
 // pf_windows2.cu
 size_t pf_win2_scratch_bytes(int n);       // records followed by the median pools
 int launch_pf_windows2(epid_ctx* ctx, cudaStream_t stream, const PfConst* cst, const FrameRef* refs, PfFrame* fr, PfWinRec* recs, PfWin* wins,

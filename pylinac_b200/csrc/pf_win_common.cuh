@@ -65,21 +65,6 @@ template <int N, int... I>
 __device__ __forceinline__ void apply_net_u64(unsigned long long (&r)[N], std::integer_sequence<int, I...>) {
     (cmpswap_u64<BatcherNet<N>::L.a[I], BatcherNet<N>::L.b[I], N>(r), ...);
 }
-template <int A, int B, int N>
-__device__ __forceinline__ void cmpswap_f64(double (&r)[N]) {
-    const double a = r[A], b = r[B];
-    r[A] = fmin(a, b);
-    r[B] = fmax(a, b);
-}
-template <int N, int... I>
-__device__ __forceinline__ void apply_net_f64(double (&r)[N], std::integer_sequence<int, I...>) {
-    (cmpswap_f64<BatcherNet<N>::L.a[I], BatcherNet<N>::L.b[I], N>(r), ...);
-}
-template <int N>
-__device__ __forceinline__ void sort_net_f64(double (&r)[N]) {
-    apply_net_f64<N>(r, std::make_integer_sequence<int, BatcherNet<N>::L.n>{});
-}
-
 template <int N>
 __device__ __forceinline__ void sort_net_u64(unsigned long long (&r)[N]) {
     apply_net_u64<N>(r, std::make_integer_sequence<int, BatcherNet<N>::L.n>{});
@@ -134,76 +119,11 @@ static __device__ __noinline__ uint2 pair_median_any(const uint16_t* __restrict_
     return make_uint2(m_lo, m_hi);
 }
 
-// ---- variants that also return the packed extreme over the rows (maximum, or minimum when want_min) of the two columns
-template <int N>
-__device__ __forceinline__ void pair_median_ext_exact(const uint16_t* __restrict__ px, int S, int t, bool want_min, uint32_t& m_lo, uint32_t& m_hi,
-                                                      uint32_t& ext2) {
-    uint32_t r[N];
-#pragma unroll
-    for (int i = 0; i < N; i++) r[i] = *reinterpret_cast<const uint32_t*>(px + i * S + 2 * t);
-    uint32_t e = r[0];
-    if (want_min) {
-#pragma unroll
-        for (int i = 1; i < N; i++) e = __vminu2(e, r[i]);
-    } else {
-#pragma unroll
-        for (int i = 1; i < N; i++) e = __vmaxu2(e, r[i]);
-    }
-    ext2 = e;
-    sort_net_u16x2<N>(r);
-    const uint32_t va = r[(N - 1) / 2], vb = r[N / 2];
-    m_lo = (va & 0xffffu) + (vb & 0xffffu);
-    m_hi = (va >> 16) + (vb >> 16);
-}
-
-template <int NRP>
-__device__ __forceinline__ void pair_median_ext_padded(const uint16_t* __restrict__ px, int S, int nr, int t, bool want_min, uint32_t& m_lo,
-                                                       uint32_t& m_hi, uint32_t& ext2) {
-    uint32_t r[NRP];
-    uint32_t e = want_min ? 0xffffffffu : 0u;
-#pragma unroll
-    for (int i = 0; i < NRP; i++) {
-        r[i] = 0xffffffffu;
-        if (i < nr) {
-            r[i] = *reinterpret_cast<const uint32_t*>(px + i * S + 2 * t);
-            e = want_min ? __vminu2(e, r[i]) : __vmaxu2(e, r[i]);
-        }
-    }
-    ext2 = e;
-    sort_net_u16x2<NRP>(r);
-    const int k1 = (nr - 1) / 2, k2 = nr / 2;
-    uint32_t va = 0, vb = 0;
-#pragma unroll
-    for (int i = 0; i < NRP; i++) {
-        if (i == k1) va = r[i];
-        if (i == k2) vb = r[i];
-    }
-    m_lo = (va & 0xffffu) + (vb & 0xffffu);
-    m_hi = (va >> 16) + (vb >> 16);
-}
-
-static __device__ __noinline__ uint3 pair_median_ext_any(const uint16_t* __restrict__ px, int S, int nr, int t, bool want_min) {
-    uint32_t m_lo = 0, m_hi = 0, e = 0;
-    switch (nr) {
-#define EPID_MED_CASE(N) case N: pair_median_ext_exact<N>(px, S, t, want_min, m_lo, m_hi, e); break;
-        EPID_MED_CASE(6) EPID_MED_CASE(7) EPID_MED_CASE(8) EPID_MED_CASE(9) EPID_MED_CASE(10) EPID_MED_CASE(11)
-        EPID_MED_CASE(12) EPID_MED_CASE(13) EPID_MED_CASE(14) EPID_MED_CASE(15) EPID_MED_CASE(16) EPID_MED_CASE(17)
-        EPID_MED_CASE(18) EPID_MED_CASE(19) EPID_MED_CASE(20) EPID_MED_CASE(21) EPID_MED_CASE(22) EPID_MED_CASE(23)
-        EPID_MED_CASE(24) EPID_MED_CASE(25) EPID_MED_CASE(26) EPID_MED_CASE(27) EPID_MED_CASE(28) EPID_MED_CASE(29)
-        EPID_MED_CASE(30) EPID_MED_CASE(31) EPID_MED_CASE(32)
-#undef EPID_MED_CASE
-        default:
-            if (nr < 6) pair_median_ext_padded<8>(px, S, nr, t, want_min, m_lo, m_hi, e);
-            else pair_median_ext_padded<32>(px, S, nr, t, want_min, m_lo, m_hi, e);      // not reached: nr <= 32 on this path
-    }
-    return make_uint3(m_lo, m_hi, e);
-}
-
 // serial FWXM analysis of one window's median profile m[0..nc) (2 * median in g units), lane-private.
 // Mirrors find_peaks(values, fwxm_height=0.5, max_number=1) on xs = (m - min) / (max - min) and scipy's _peak_widths.
 // returns valid (1), 0 = no peak / flat (the caller raises EPID_PF_WINDOW_NO_PEAK)
 template <int ST = 1>
-__device__ inline int lb_window_fwxm(const uint32_t* __restrict__ mbase, int nc, double& out_l, double& out_r) {
+__device__ inline int window_fwxm(const uint32_t* __restrict__ mbase, int nc, double& out_l, double& out_r) {
     auto M = [&](int j) { return mbase[j * ST]; };
     // one branch-light pass (the lanes of the warp -- one window each -- stay in lockstep): min, max and the two highest local
     // maxima (scipy _local_maxima_1d: rise, plateau, fall; midpoint of the plateau), key = height << 8 | position

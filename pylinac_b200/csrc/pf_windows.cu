@@ -18,11 +18,7 @@
 // The CTA's shared memory is split into per-warp slots sized for the frame's largest window (all 16 warps for ordinary
 // windows, fewer for very wide ones).  Windows that do not fit at all (nc > 256, nr > 64) are marked valid = -1 and picked up by the
 // generic kernel (k_pf_windows in pf.cu) launched right after in "todo" mode.
-#include <cstdio>
-#include <cstdlib>
-
 #include "pf_common.cuh"
-#include "tma.cuh"
 #include "pf_win_common.cuh"
 
 namespace epid {
@@ -90,8 +86,6 @@ __device__ __forceinline__ void row_std_stats(const uint16_t* __restrict__ px, i
     sd_med = (nr & 1) ? med_a : (med_a + med_b) / 2.0;
 }
 
-__device__ inline bool pf_leafband_ok(const PfConst& c, const PfFrame& f, const FrameRef& fr, int lane);   // defined with k_pf_leafband below
-
 __global__ void __launch_bounds__(W2_WARPS * 32, 2)
 k_pf_windows_fast(const PfConst* __restrict__ cc, const FrameRef* __restrict__ frames, PfFrame* fr, PfWin* __restrict__ wins) {
     extern __shared__ __align__(16) unsigned char smraw[];
@@ -106,7 +100,6 @@ k_pf_windows_fast(const PfConst* __restrict__ cc, const FrameRef* __restrict__ f
     if (wid == 0) {
         // slot size from the frame's largest possible window (other CTAs may change f.status meanwhile: read it once)
         const int st = f.status;
-        const bool leafband = pf_leafband_ok(c, f, frames[fi], lane);     // that kernel owns this frame's windows
         double lw = 0.0;
         for (int i = lane; i < f.n_inview; i += 32) lw = fmax(lw, c.p.leaf_width_mm[f.inview[i]] * dpmm);
         lw = warp_max(lw);
@@ -118,7 +111,7 @@ k_pf_windows_fast(const PfConst* __restrict__ cc, const FrameRef* __restrict__ f
             int stage_b = max(nr_max * s_max * 2, nc_max * 8);
             stage_b = (stage_b + 15) & ~15;
             const int slot = stage_b + ((nc_max * 4 + 15) & ~15);
-            s_geo[0] = (leafband || f.win2) ? -1 : st;     // another window kernel owns this frame
+            s_geo[0] = f.win2 ? -1 : st;     // the two-kernel window path owns this frame
             s_geo[1] = slot;
             s_geo[2] = stage_b;
             s_geo[3] = nc_max > W2_MAXNC + 2 ? 0 : min(W2_WARPS, W2_POOL / slot);
@@ -478,344 +471,10 @@ k_pf_windows_fast(const PfConst* __restrict__ cc, const FrameRef* __restrict__ f
     }
 }
 
-// =====================================================================================================================
-// Leaf-band kernel: one CTA works on one LEAF of one frame at a time -- all pickets of that leaf together.
-//
-// The windows of a leaf are column ranges of the same band of rows, so the band is brought into shared memory once (one TMA bulk
-// copy per row, raw pixels, completion on an mbarrier) and every phase keeps all lanes busy:
-//   P1  threads own (row, picket) pairs: sum / sum of squares / min / max of the row inside the picket's window.  The variance
-//       numerator nc * S2 - S1^2 is an exact integer and is invariant under the frame's ground / inversion map, so raw pixels do;
-//   P2  threads own words (pairs of columns) of the band: median over the rows by the same register sorting networks as the
-//       per-window kernel; the median commutes with the monotone ground / inversion map, which is applied to the result.  Columns
-//       shared by neighbouring windows are computed once;
-//   P1b a warp per picket (lanes = rows): window maximum, max(std) and median(std) -- ranked on the integer variance numerators,
-//       only the two or three selected rows see a square root -- and the validity decision of _is_mlc_peak_in_window;
-//   P3  ONE warp, lanes = pickets: the 1-D FWXM analysis of each window's median profile, serial per lane on the integer medians
-//       (fp64 only for the prominence, the half-height threshold and the two interpolations).  While it runs, the other warps
-//       already work on the next leaf (its band was requested as soon as P2 released the buffer); the P3 warp rotates.
-// Results are bit-identical to k_pf_windows_fast (same integer quantities, same fp64 expressions); frames the band layout does
-// not cover (Left-Right orientation, unaligned pitch, leaves wider than 32 rows, ...) are left to that kernel: both kernels take
-// the decision with pf_leafband_ok().
-constexpr int LB_WARPS = 8;
-constexpr int LB_THREADS = LB_WARPS * 32;
-constexpr int LB_BAND_BYTES = 30 * 1024;
-constexpr int LB_MAXJ = 704;           // band columns (aligned grid) that have a median slot
-constexpr int LB_MAXP = 16;           // pickets per frame on this path
-constexpr int LB_MAXLEAVES = 32;      // leaves per work item
-constexpr int LB_LAG = 3;             // leaves a warp sits out after taking a leaf's 1-D analysis (P3)
-constexpr int LB_RING = LB_LAG + 1;   // median-profile buffers in flight
-constexpr int LB_MAXNR = 32;
-constexpr int LB_CHUNKS = 4;           // work items per frame (groups of leaves)
-
-__device__ __forceinline__ int lb_row_stride_bytes(int nvec) { return (nvec | 1) * 16; }   // odd vector count: rows start in different banks
-
-// warp-collective: may this frame's windows be processed by the leaf-band kernel?  (same answer in both window kernels)
-__device__ inline bool pf_leafband_ok(const PfConst& c, const PfFrame& f, const FrameRef& fr, int lane) {
-    if (!c.leafband) return false;
-    const int st = f.status;
-    const double sp = f.spacing;
-    bool ok = st == EPID_PF_OK && f.orientation == 0 && (fr.pitch & 7) == 0 && f.n_pickets >= 1 && f.n_pickets <= LB_MAXP &&
-              sp == sp && sp >= 2.0 && sp < 254.0 && f.n_inview > 0 && (f.n_inview + LB_CHUNKS - 1) / LB_CHUNKS <= LB_MAXLEAVES;
-    if (!ok) return false;
-    const double dpmm = c.p.dpmm;
-    int nr_max = 0, nr_min = 1 << 30;
-    for (int i = lane; i < f.n_inview; i += 32) {
-        const int leaf = f.inview[i];
-        const double lw_px = c.p.leaf_width_mm[leaf] * dpmm;
-        const double lc_px = c.p.leaf_center_mm[leaf] * dpmm + (double)c.H / 2.0;
-        const int b0 = max((int)(lc_px - lw_px / 2.0), 0), b1 = min((int)(lc_px + lw_px / 2.0), c.H);
-        nr_max = max(nr_max, b1 - b0);
-        nr_min = min(nr_min, b1 - b0);
-    }
-    nr_max = warp_max(nr_max);
-    nr_min = warp_min(nr_min);
-    // the band: the columns between the first and the last picket window (+ up to 7 pixels of alignment on either side)
-    int a0 = c.W, a1 = 0;
-    if (lane < f.n_pickets) {
-        const double pidx = (double)f.picket_idx[lane];
-        a0 = max((int)(pidx - sp / 2.0), 0);
-        a1 = min((int)(pidx + sp / 2.0), c.W);
-        if (a1 <= a0) { a0 = c.W; a1 = 0; }
-    }
-    const int cmin = warp_min(a0), cmax = warp_max(a1);
-    const int cols = cmax > cmin ? cmax - cmin + 14 : 16;
-    const int nvec = (cols + 7) / 8;
-    return nr_min >= 1 && nr_max <= LB_MAXNR && nvec * 8 + 2 <= LB_MAXJ && nr_max * lb_row_stride_bytes(nvec) <= LB_BAND_BYTES;
-}
-
-struct LbCols {       // the same for every leaf of a frame: the columns the picket windows cover
-    int cs, nvec;      // first aligned-grid column of the band (view coordinates, may be < 0), 8-pixel vectors per row
-    int jlo, jhi;      // band-relative column range that belongs to some window
-    int RS;            // row stride in bytes
-};
-
-__device__ __forceinline__ void lb_window_cols(const PfFrame& f, int W, int pk, int& a0, int& a1) {
-    const double pidx = (double)f.picket_idx[pk], spacing = f.spacing;
-    a0 = max((int)(pidx - spacing / 2.0), 0);      // _get_mlc_window (picketfence.py:859-886): int() truncates toward zero
-    a1 = min((int)(pidx + spacing / 2.0), W);
-}
-
-__device__ __forceinline__ void lb_leaf_rows(const PfConst& c, const PfFrame& f, int li, int& b0, int& nr) {
-    const int leaf = f.inview[li];
-    const double lw_px = c.p.leaf_width_mm[leaf] * c.p.dpmm;
-    const double lc_px = c.p.leaf_center_mm[leaf] * c.p.dpmm + (double)c.H / 2.0;
-    b0 = max((int)(lc_px - lw_px / 2.0), 0);
-    nr = min((int)(lc_px + lw_px / 2.0), c.H) - b0;
-}
-
-__device__ __forceinline__ void lb_named_bar(int id, int nthreads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
-
-__global__ void __launch_bounds__(LB_THREADS, 4)
-k_pf_leafband(const PfConst* __restrict__ cc, const FrameRef* __restrict__ frames, PfFrame* fr, PfWin* __restrict__ wins, int n) {
-    extern __shared__ __align__(128) unsigned char lbraw[];
-    unsigned char* band = lbraw;
-    uint32_t* s_m2 = reinterpret_cast<uint32_t*>(lbraw + LB_BAND_BYTES);                         // [LB_RING][LB_MAXJ]
-    unsigned long long* s_num = reinterpret_cast<unsigned long long*>(s_m2 + LB_RING * LB_MAXJ); // [LB_MAXP * 32]
-    uint32_t* s_ext = reinterpret_cast<uint32_t*>(s_num + LB_MAXP * 32);                         // [LB_MAXP * 32]: max << 16 | min
-    int* s_valid = reinterpret_cast<int*>(s_ext + LB_MAXP * 32);                                 // [LB_RING][LB_MAXP]
-    __shared__ __align__(8) unsigned long long s_bar;
-    __shared__ int s_ok;
-    __shared__ int s_a0[LB_MAXP], s_a1[LB_MAXP];
-    __shared__ double s_pval[LB_MAXP];
-    __shared__ short s_b0[LB_MAXLEAVES], s_nr[LB_MAXLEAVES];
-    __shared__ LbCols s_cols;
-    const PfConst& c = *cc;
-    const int tid = threadIdx.x, wid = tid >> 5, lane = tid & 31;
-    const int W = c.W, H = c.H;
-    const double height_thr = c.p.height_threshold, edge_thr = c.p.edge_threshold;
-    const int sag = c.p.sag_px;
-    if (tid == 0) { mbar_init(smem_u32(&s_bar), 1); mbar_fence_init(); }
-    __syncthreads();
-    const uint32_t bar = smem_u32(&s_bar);
-    uint32_t phase = 0;          // parity of the band transfer of the next leaf (advanced by every warp for every leaf)
-    const int nitems = n * LB_CHUNKS;
-    for (int item = blockIdx.x; item < nitems; item += gridDim.x) {
-        const int fi = item / LB_CHUNKS, ch = item - fi * LB_CHUNKS;
-        PfFrame& f = fr[fi];
-        const FrameRef frf = frames[fi];
-        const int mis = (int)((reinterpret_cast<uintptr_t>(frf.origin) >> 1) & 7);
-        __syncthreads();        // the previous item is finished in every warp (its P3 stragglers included): shared state is free
-        if (wid == 0) {
-            const bool ok = pf_leafband_ok(c, f, frf, lane);
-            if (ok) {
-                // everything the per-leaf loop needs from global memory, once per item: window columns, picket heights, leaf rows
-                int a0 = W, a1 = 0;
-                if (lane < f.n_pickets) {
-                    lb_window_cols(f, W, lane, a0, a1);
-                    s_a0[lane] = a0;
-                    s_a1[lane] = a1;
-                    s_pval[lane] = f.picket_val[lane];
-                    if (a1 <= a0) { a0 = W; a1 = 0; }
-                }
-                int cmin = warp_min(a0), cmax = warp_max(a1);
-                if (cmax <= cmin) { cmin = 0; cmax = 8; }
-                const int per = (f.n_inview + LB_CHUNKS - 1) / LB_CHUNKS;
-                if (lane < per && ch * per + lane < f.n_inview) {
-                    int b0, nr;
-                    lb_leaf_rows(c, f, ch * per + lane, b0, nr);
-                    s_b0[lane] = (short)b0;
-                    s_nr[lane] = (short)nr;
-                }
-                if (lane == 0) {
-                    LbCols g;
-                    g.cs = cmin - ((cmin + mis) & 7);
-                    const int ce = cmax + ((8 - ((cmax + mis) & 7)) & 7);
-                    g.nvec = (ce - g.cs) >> 3;
-                    g.jlo = cmin - g.cs;
-                    g.jhi = cmax - g.cs;
-                    g.RS = lb_row_stride_bytes(g.nvec);
-                    s_cols = g;
-                }
-            }
-            if (lane == 0) s_ok = ok ? 1 : 0;
-        }
-        __syncthreads();
-        if (!s_ok) continue;
-        const int np = f.n_pickets;
-        const int per = (f.n_inview + LB_CHUNKS - 1) / LB_CHUNKS;
-        const int l0 = ch * per, l1 = min(f.n_inview, l0 + per);
-        if (l0 >= l1) continue;
-        const LbCols g = s_cols;
-        const int inv = f.inv;
-        const uint32_t mn = f.mn, mx = f.mx;
-        const double Dd = (double)f.D;
-        auto request_band = [&](int b0, int nr) {            // one worker warp, after the barrier that released the band buffer
-            if (lane == 0) mbar_expect_tx(bar, (uint32_t)nr * (uint32_t)g.nvec * 16u);
-            __syncwarp();
-            if (lane < nr) {
-                int row = b0 + lane - sag;
-                if (sag) { row %= H; if (row < 0) row += H; }
-                tma_load_1d(smem_u32(band + (size_t)lane * g.RS), frf.origin + ((ptrdiff_t)row * frf.pitch + g.cs), (uint32_t)g.nvec * 16u, bar);
-            }
-        };
-        if (wid == 0) request_band(s_b0[0], s_nr[0]);
-        // Leaf j's 1-D analysis (P3) is done by warp j % LB_WARPS, which then sits out the next LB_LAG leaves entirely (no work, no
-        // barriers): the other warps carry on, synchronised by named barriers over exactly the warps that take part in a leaf.
-        for (int j = 0; j < l1 - l0; j++) {
-            const int li = l0 + j;
-            const int nout = min(j, LB_LAG);
-            bool out = false;
-            int widx = 0;
-#pragma unroll
-            for (int v = 0; v < LB_WARPS; v++) {
-                bool o = false;
-#pragma unroll
-                for (int d = 1; d <= LB_LAG; d++) o = o || (d <= nout && ((j - d) % LB_WARPS) == v);
-                if (v == wid) out = o;
-                else if (v < wid && !o) widx++;
-            }
-            const uint32_t ph = phase;
-            phase ^= 1u;
-            const int nwork = (LB_WARPS - nout) * 32;
-            const int bid = 1 + 2 * (j & 3);                  // barrier ids of this leaf (a 4-leaf cycle > LB_LAG)
-            // the warp whose sit-out ends with this leaf attends its B2: from there on it is in step with the others again (the
-            // band transfer it waits for next has been requested, num / ext and the oldest median buffer are free)
-            const int nb2 = nwork + (j >= LB_LAG ? 32 : 0);
-            if (out) {
-                if (j >= LB_LAG && wid == (j - LB_LAG) % LB_WARPS) lb_named_bar(bid + 1, nb2);
-                continue;
-            }
-            const int q = j % LB_RING;
-            uint32_t* m2 = s_m2 + q * LB_MAXJ;
-            int* valid = s_valid + q * LB_MAXP;
-            const int nr = s_nr[j];
-            mbar_wait(bar, ph);
-            // ---- P1: (row, picket) sums on the raw pixels; tasks are dealt from the first worker thread upwards
-            for (int t = widx * 32 + lane; t < nr * np; t += nwork) {
-                const int r = t / np, pk = t - r * np;
-                const int a0 = s_a0[pk], a1 = s_a1[pk];
-                unsigned long long numv = 0;
-                uint32_t e = 0x0000ffffu;
-                if (a1 > a0) {
-                    const unsigned char* rowp = band + (size_t)r * g.RS;
-                    int j0 = a0 - g.cs, j1 = a1 - g.cs;
-                    uint32_t s1 = 0, vmx = 0, vmn = 0xffffu;
-                    unsigned long long s2 = 0;
-                    if (j0 & 1) {
-                        const uint32_t v = *reinterpret_cast<const uint16_t*>(rowp + 2 * j0);
-                        s1 += v; s2 += (unsigned long long)v * v; vmx = max(vmx, v); vmn = min(vmn, v);
-                        j0++;
-                    }
-                    if (j1 & 1) {
-                        const uint32_t v = *reinterpret_cast<const uint16_t*>(rowp + 2 * (j1 - 1));
-                        s1 += v; s2 += (unsigned long long)v * v; vmx = max(vmx, v); vmn = min(vmn, v);
-                        j1--;
-                    }
-                    uint32_t mx2 = 0, mn2 = 0xffffffffu;
-                    const uint32_t* wp = reinterpret_cast<const uint32_t*>(rowp);
-#pragma unroll 4
-                    for (int w = j0 >> 1; w < (j1 >> 1); w++) {
-                        const uint32_t x = wp[w];
-                        const uint32_t lo = x & 0xffffu, hi = x >> 16;
-                        s1 = __dp2a_lo(x, 0x0101u, s1);
-                        s2 += (unsigned long long)lo * lo;
-                        s2 += (unsigned long long)hi * hi;
-                        mx2 = __vmaxu2(mx2, x);
-                        mn2 = __vminu2(mn2, x);
-                    }
-                    if (j1 > j0) {
-                        vmx = max(vmx, max(mx2 & 0xffffu, mx2 >> 16));
-                        vmn = min(vmn, min(mn2 & 0xffffu, mn2 >> 16));
-                    }
-                    const unsigned long long ncl = (unsigned long long)(a1 - a0);
-                    numv = ncl * s2 - (unsigned long long)s1 * s1;
-                    e = (vmx << 16) | vmn;
-                }
-                s_num[pk * 32 + r] = numv;
-                s_ext[pk * 32 + r] = e;
-            }
-            // ---- P2: 2 * median over the rows for every pair of band columns that some window uses; tasks are dealt from the
-            //      LAST worker thread downwards, so that the warps P1 left idle take them first
-            {
-                const uint16_t* px = reinterpret_cast<const uint16_t*>(band);
-                const int S = g.RS >> 1;
-                for (int t = (g.jlo >> 1) + (nwork - 1 - (widx * 32 + lane)); t < ((g.jhi + 1) >> 1); t += nwork) {
-                    const uint2 mm = pair_median_any(px, S, nr, t);
-                    m2[2 * t] = inv ? 2u * mx - mm.x : mm.x - 2u * mn;
-                    m2[2 * t + 1] = inv ? 2u * mx - mm.y : mm.y - 2u * mn;
-                }
-            }
-            lb_named_bar(bid, nwork);              // B1: band released, num / ext / m2 of this leaf complete
-            // request the next leaf's band right away (the same buffer): it lands while P1b / P3 run
-            if (j + 1 < l1 - l0 && widx == 0) request_band(s_b0[j + 1], s_nr[j + 1]);
-            // ---- P1b: _is_mlc_peak_in_window (picketfence.py:847-857), a warp per picket, lanes = rows
-            for (int pk = widx; pk < np; pk += LB_WARPS - nout) {
-                const int nc = s_a1[pk] - s_a0[pk];
-                int ok = 0;
-                if (nc > 0) {
-                    const unsigned long long key = lane < nr ? s_num[pk * 32 + lane] : 0ull;
-                    const uint32_t e = lane < nr ? s_ext[pk * 32 + lane] : 0x0000ffffu;
-                    const uint32_t vmx = __reduce_max_sync(0xffffffffu, e >> 16), vmn = __reduce_min_sync(0xffffffffu, e & 0xffffu);
-                    const uint32_t gmax = inv ? mx - vmn : vmx - mn;
-                    // rank of every row's variance numerator (ties by row index), the largest numerator
-                    int rank = 0;
-                    unsigned long long kmax = 0;
-                    for (int t = 0; t < nr; t++) {
-                        const unsigned long long o = __shfl_sync(0xffffffffu, key, t);
-                        if (o < key || (o == key && t < lane)) rank++;
-                        kmax = o > kmax ? o : kmax;
-                    }
-                    const int k1 = (nr - 1) / 2, k2 = nr / 2;
-                    const unsigned ba = __ballot_sync(0xffffffffu, lane < nr && rank == k1);
-                    const unsigned bb = __ballot_sync(0xffffffffu, lane < nr && rank == k2);
-                    const unsigned long long ka = __shfl_sync(0xffffffffu, key, __ffs(ba) - 1);
-                    const unsigned long long kb = __shfl_sync(0xffffffffu, key, __ffs(bb) - 1);
-                    const double dn = (double)nc * Dd;
-                    const double sd_max = sqrt((double)kmax) / dn;
-                    const double sa = sqrt((double)ka) / dn, sb = sqrt((double)kb) / dn;
-                    const double sd_med = (nr & 1) ? sa : (sa + sb) / 2.0;
-                    const bool above = ((double)gmax / Dd) > height_thr * s_pval[pk];
-                    const bool not_edge = sd_max < edge_thr * sd_med;
-                    ok = (above && not_edge) ? 1 : 0;
-                } else if (lane == 0) {
-                    f.status = EPID_PF_WINDOW_NO_PEAK;       // empty slice: np.max raises ValueError in the reference
-                }
-                if (lane == 0) valid[pk] = ok;
-            }
-            lb_named_bar(bid + 1, nb2);            // B2: valid[] complete (and num / ext free for the next leaf)
-            // ---- P3: lanes = pickets, by the warp whose turn it is; it rejoins LB_LAG leaves later
-            if (wid == j % LB_WARPS && lane < np) {
-                PfWin& outw = wins[((size_t)fi * PF_L + li) * PF_P + lane];
-                if (!valid[lane]) {
-                    outw.valid = 0; outw.l = 0; outw.r = 0;
-                } else {
-                    double l = 0, r = 0;
-                    const int v = lb_window_fwxm(m2 + (s_a0[lane] - g.cs), s_a1[lane] - s_a0[lane], l, r);
-                    outw.valid = v;
-                    if (v) { outw.l = l; outw.r = r; }
-                    else f.status = EPID_PF_WINDOW_NO_PEAK;
-                }
-            }
-        }
-    }
-}
-
-int launch_pf_leafband(epid_ctx* ctx, cudaStream_t stream, const PfConst* cst, const FrameRef* refs, PfFrame* fr, PfWin* wins, int n) {
-    const size_t smem = LB_BAND_BYTES + sizeof(uint32_t) * LB_RING * LB_MAXJ + sizeof(unsigned long long) * LB_MAXP * 32 +
-                        sizeof(uint32_t) * LB_MAXP * 32 + sizeof(int) * LB_RING * LB_MAXP + 64;
-    if (ctx->smem_optin.find((const void*)k_pf_leafband) == ctx->smem_optin.end()) {
-        EPID_SMEM_OPT_IN(ctx, k_pf_leafband, smem);
-        EPID_CUDA(cudaFuncSetAttribute(k_pf_leafband, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        if (getenv("EPID_DEBUG")) {
-            int nb = 0;
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_pf_leafband, LB_THREADS, smem);
-            fprintf(stderr, "[epid] k_pf_leafband: %zu B dynamic shared memory, %d CTAs / SM\n", smem, nb);
-        }
-    }
-    const int nitems = n * LB_CHUNKS;
-    const int grid = nitems < 4 * ctx->sm_count ? nitems : 4 * ctx->sm_count;
-    k_pf_leafband<<<grid, LB_THREADS, smem, stream>>>(cst, refs, fr, wins, n);
-    ctx->launches++;
-    EPID_CUDA(cudaGetLastError());
-    return EPID_OK;
-}
-
 int launch_pf_windows_fast(epid_ctx* ctx, cudaStream_t stream, const PfConst* cst, const FrameRef* refs, PfFrame* fr, PfWin* wins, int n) {
     const size_t smem = W2_POOL;
     EPID_SMEM_OPT_IN(ctx, k_pf_windows_fast, smem);
-    static int gx = 0;
-    if (gx == 0) { const char* e = getenv("EPID_W2_GRID"); gx = e ? atoi(e) : W2_GRID_X; if (gx < 1 || gx > 64) gx = W2_GRID_X; }
-    dim3 grid(gx, n);
+    dim3 grid(W2_GRID_X, n);
     k_pf_windows_fast<<<grid, W2_WARPS * 32, smem, stream>>>(cst, refs, fr, wins);
     ctx->launches++;
     EPID_CUDA(cudaGetLastError());

@@ -19,15 +19,12 @@
 //           pool contiguously (columns shared by overlapping windows are computed once).
 //   k_pf_win_fwxm      thread per window, 32 windows of a warp in lock step: _is_mlc_peak_in_window from the three numerators and
 //       the window maximum (same fp64 expressions as the reference), then the serial integer FWXM analysis of the median profile
-//       (lb_window_fwxm: fp64 only for the prominence, the half-height level and the two interpolations).  The profiles are
+//       (window_fwxm: fp64 only for the prominence, the half-height level and the two interpolations).  The profiles are
 //       transposed through shared memory ([sample][window], stride 33): coalesced pool reads, conflict-free per-thread walks.
 //
 // Results are bit-identical to k_pf_windows_fast (same integer quantities, same fp64 expressions; tests/test_gpu_pf.py compares
 // them).  Frames this path does not cover (Left-Right orientation, unaligned pitch, windows wider than 64 samples or taller than
 // 32 rows, more than 1024 windows) are left to k_pf_windows_fast: this kernel sets PfFrame.win2 for the frames it takes.
-#include <cstdio>
-#include <cstdlib>
-
 #include "pf_common.cuh"
 #include "pf_win_common.cuh"
 #include "tma.cuh"
@@ -35,8 +32,9 @@
 namespace epid {
 
 constexpr int WA_WARPS = 8;
-constexpr int WA_SLOT_BIG = 6656;      // bytes per staging slot: 26 rows x 256 B (two 51-sample windows of a 10 mm leaf at 2.56 px/mm), 2 CTAs / SM
-constexpr int WA_SLOT_SMALL = 4416;    // 13 rows x 336 B (three such windows of a 5 mm leaf), 3 CTAs / SM
+// bytes per staging slot: 13 rows x 336 B (three 51-sample windows of a 5 mm leaf at 2.56 px/mm), 3 CTAs / SM.  Measured against
+// 6656-byte slots (26 rows x 256 B, 2 CTAs / SM): 0.296 vs 0.317 ms per 512 frames
+constexpr int WA_SLOT = 4416;
 constexpr int WA_GRID_X = 4;           // CTAs per frame
 constexpr int WA_GMAX = 4;             // pickets per task
 constexpr int WA_KMAX = 4;             // rows per lane in P1: ceil(32 rows / (32 lanes / 4 pickets))
@@ -51,8 +49,7 @@ struct W2Geo {
     int gtot[WA_GMAX + 1];      // median-pool samples of one leaf when pickets are taken g at a time
 };
 
-template <int WA_SLOT, int MINB>
-__global__ void __launch_bounds__(WA_WARPS * 32, MINB)
+__global__ void __launch_bounds__(WA_WARPS * 32, 3)
 k_pf_win_medians(const PfConst* __restrict__ cc, const FrameRef* __restrict__ frames, PfFrame* fr, PfWinRec* __restrict__ recs,
                  uint32_t* __restrict__ pools) {
     extern __shared__ __align__(128) unsigned char smraw[];          // WA_WARPS x 2 slots
@@ -421,7 +418,7 @@ k_pf_win_fwxm(const PfConst* __restrict__ cc, PfFrame* fr, const PfWinRec* __res
     __syncwarp();
     if (run) {
         double l = 0, r = 0;
-        const int v = lb_window_fwxm<WB_ST>(buf + lane, my_nc, l, r);
+        const int v = window_fwxm<WB_ST>(buf + lane, my_nc, l, r);
         out.valid = v;
         if (v) { out.l = l; out.r = r; }
         else f.status = EPID_PF_WINDOW_NO_PEAK;
@@ -436,19 +433,9 @@ size_t pf_win2_scratch_bytes(int n) {
 int launch_pf_windows2(epid_ctx* ctx, cudaStream_t stream, const PfConst* cst, const FrameRef* refs, PfFrame* fr, PfWinRec* recs, PfWin* wins,
                        int n, PfTimers* tm) {
     uint32_t* pools = reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(recs) + ((sizeof(PfWinRec) * (size_t)n * PF_W2_WCAP + 255) / 256) * 256);
-    static int gx = 0;
-    if (gx == 0) { const char* e = getenv("EPID_WA_GRID"); gx = e ? atoi(e) : WA_GRID_X; if (gx < 1 || gx > 64) gx = WA_GRID_X; }
-    static int small_slots = -1;
-    if (small_slots < 0) { const char* e = getenv("EPID_WA_SMALL"); small_slots = e ? atoi(e) : 1; }     // measured: 0.296 vs 0.317 ms per 512 frames
-    if (small_slots == 1) {
-        const size_t smem = (size_t)WA_WARPS * 2 * WA_SLOT_SMALL;
-        EPID_SMEM_OPT_IN(ctx, (k_pf_win_medians<WA_SLOT_SMALL, 3>), smem);
-        k_pf_win_medians<WA_SLOT_SMALL, 3><<<dim3(gx, n), WA_WARPS * 32, smem, stream>>>(cst, refs, fr, recs, pools);
-    } else {
-        const size_t smem = (size_t)WA_WARPS * 2 * WA_SLOT_BIG;
-        EPID_SMEM_OPT_IN(ctx, (k_pf_win_medians<WA_SLOT_BIG, 2>), smem);
-        k_pf_win_medians<WA_SLOT_BIG, 2><<<dim3(gx, n), WA_WARPS * 32, smem, stream>>>(cst, refs, fr, recs, pools);
-    }
+    const size_t smem = (size_t)WA_WARPS * 2 * WA_SLOT;
+    EPID_SMEM_OPT_IN(ctx, k_pf_win_medians, smem);
+    k_pf_win_medians<<<dim3(WA_GRID_X, n), WA_WARPS * 32, smem, stream>>>(cst, refs, fr, recs, pools);
     ctx->launches++;
     if (tm) { int rc = tm->mark(stream, PF_STAGE_WIN_MEDIANS); if (rc != EPID_OK) return rc; }
     k_pf_win_fwxm<<<dim3(PF_W2_WCAP / WB_THREADS, n), WB_THREADS, 0, stream>>>(cst, fr, recs, pools, wins);

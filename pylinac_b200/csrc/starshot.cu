@@ -759,7 +759,7 @@ extern "C" int32_t epid_starshot_analyze(epid_ctx* ctx, const epid_batch* frames
     gc.ranks[0] = hc.p90.prev; gc.ranks[1] = hc.p90.next;
     gc.ranks[2] = nc - 1 - hc.p90.next; gc.ranks[3] = nc - 1 - hc.p90.prev;
     gc.box = 0;
-    rc = launch_frame_stats(ctx, st, gc, d_rc, nullptr, n, d_sc, nullptr, nullptr);
+    rc = launch_frame_stats(ctx, st, gc, d_rc, n, d_sc, nullptr, nullptr);
     if (rc != EPID_OK) return rc;
     {
         const int n_max = hc.cw > hc.ch ? hc.cw : hc.ch;

@@ -14,8 +14,6 @@
 // a frame share one value; that is detected exactly (the decoded bin total then differs from the pixel count)
 // and the frame is re-run by the MODE 1 variant (32-bit counters over value>>1 plus a second pass resolving
 // the low bit), so results are always exact.
-#include <cstdlib>
-
 #include "stats.cuh"
 
 namespace epid {
@@ -70,7 +68,7 @@ __device__ __forceinline__ void block_scan_excl_1024(uint32_t v, uint32_t* s_war
 // MODE 0: packed u16 counters, all 65536 bins.  MODE 1: u32 counters over (v >> 1), low bit resolved by a 2nd pass.
 template <int MODE>
 __global__ void __launch_bounds__(STATS_THREADS, 1)
-k_frame_stats(const StatsGeom g, const FrameRef* __restrict__ frames, const int* __restrict__ out_index, int nframes,
+k_frame_stats(const StatsGeom g, const FrameRef* __restrict__ frames, int nframes,
               FrameStats* __restrict__ stats, uint32_t* __restrict__ rowsum_out, uint32_t* __restrict__ colsum_out) {
     extern __shared__ uint32_t smem[];
     uint32_t* hist = smem;                                   // HIST_WORDS
@@ -86,8 +84,7 @@ k_frame_stats(const StatsGeom g, const FrameRef* __restrict__ frames, const int*
     const bool active_grp = grp < g.groups;
 
     for (int fi = blockIdx.x; fi < nframes; fi += gridDim.x) {
-        const int slot = out_index ? out_index[fi] : fi;
-        if (MODE == 1 && stats[slot].overflow == 0) continue;
+        if (MODE == 1 && stats[fi].overflow == 0) continue;
         const FrameRef fr = frames[fi];
         const uint16_t* __restrict__ f = fr.origin;
         const int pitch = fr.pitch;
@@ -215,11 +212,11 @@ k_frame_stats(const StatsGeom g, const FrameRef* __restrict__ frames, const int*
                 const int ac = x + mis;  // position inside the per-row vector grid
                 uint32_t s = 0;
                 for (int gg = 0; gg < g.groups; gg++) s += colpart[(gg * g.vprp) * 8 + ac];
-                colsum_out[(size_t)slot * g.W + x] = s;
+                colsum_out[(size_t)fi * g.W + x] = s;
             }
         }
         if (rowsum_out)
-            for (int y = tid; y < g.H; y += STATS_THREADS) rowsum_out[(size_t)slot * g.H + y] = rowsum_sm[y];
+            for (int y = tid; y < g.H; y += STATS_THREADS) rowsum_out[(size_t)fi * g.H + y] = rowsum_sm[y];
 
         // ---- order statistics from the histogram
         uint32_t cnt = 0;
@@ -284,7 +281,7 @@ k_frame_stats(const StatsGeom g, const FrameRef* __restrict__ frames, const int*
             __syncthreads();
         }
         if (tid == 0) {
-            FrameStats& o = stats[slot];
+            FrameStats& o = stats[fi];
             o.mn = s_misc[0];
             o.mx = s_misc[1];
             o.npix = npix;
@@ -807,7 +804,7 @@ static void launch_inv_stream(cudaStream_t st, bool cols, const StatsGeom& g, co
 int launch_frame_stats_inversion(epid_ctx* ctx, cudaStream_t stream, const StatsGeom& g, const FrameRef* d_frames, int n, FrameStats* d_stats,
                                  uint32_t* d_rowsum, uint32_t* d_colsum) {
     if (ctx->stats_exact || g.nranks != 6 || g.box > 0 || g.W > 2040 || g.H < IV_SAMPLE_ROWS || g.W < 8)
-        return launch_frame_stats(ctx, stream, g, d_frames, nullptr, n, d_stats, d_rowsum, d_colsum);
+        return launch_frame_stats(ctx, stream, g, d_frames, n, d_stats, d_rowsum, d_colsum);
     const int nvec = (g.W + 7 + 7) / 8;
     const int vpl = (nvec + 31) / 32;
     const int wa = vpl * 32 * 8;
@@ -844,7 +841,7 @@ int launch_frame_stats_inversion(epid_ctx* ctx, cudaStream_t stream, const Stats
     ctx->stats_uncertified += m;
     if (m > 0) {       // exact order statistics for the frames whose decision could not be certified
         k_inv_gather_refs<<<(m + 127) / 128, 128, 0, stream>>>(d_frames, list + 1, m, refs2);
-        int rc = launch_frame_stats(ctx, stream, g, refs2, nullptr, m, tmp, nullptr, nullptr);
+        int rc = launch_frame_stats(ctx, stream, g, refs2, m, tmp, nullptr, nullptr);
         if (rc != EPID_OK) return rc;
         k_inv_scatter_ostat<<<(m + 127) / 128, 128, 0, stream>>>(tmp, list + 1, m, d_stats);
         ctx->launches += 2;
@@ -858,19 +855,17 @@ static size_t stats_smem_bytes(const StatsGeom& g) {
 }
 
 int launch_frame_stats(epid_ctx* ctx, cudaStream_t stream, const StatsGeom& g, const FrameRef* d_frames,
-                       const int* d_out_index, int n, FrameStats* d_stats, uint32_t* d_rowsum, uint32_t* d_colsum) {
-    // multi-CTA histogram path for every view it covers (d_out_index is not used by any caller of that path)
-    static int v1 = -1;
-    if (v1 < 0) { const char* e = getenv("EPID_STATS_V1"); v1 = e ? atoi(e) : 0; }
-    if (!v1 && !d_out_index && g.W <= 2040 && g.nranks <= STATS_MAX_RANKS)
+                       int n, FrameStats* d_stats, uint32_t* d_rowsum, uint32_t* d_colsum) {
+    // multi-CTA histogram path for every view it covers
+    if (g.W <= 2040 && g.nranks <= STATS_MAX_RANKS)
         return launch_frame_stats_v2(ctx, stream, g, d_frames, n, d_stats, d_rowsum, d_colsum);
     const size_t smem = stats_smem_bytes(g);
     EPID_SMEM_OPT_IN(ctx, k_frame_stats<0>, 220 * 1024);
     EPID_SMEM_OPT_IN(ctx, k_frame_stats<1>, 220 * 1024);
     const int grid = n < ctx->sm_count ? n : ctx->sm_count;
-    k_frame_stats<0><<<grid, STATS_THREADS, smem, stream>>>(g, d_frames, d_out_index, n, d_stats, d_rowsum, d_colsum);
+    k_frame_stats<0><<<grid, STATS_THREADS, smem, stream>>>(g, d_frames, n, d_stats, d_rowsum, d_colsum);
     // exact fallback for frames whose packed counters overflowed (CTAs of other frames exit at once)
-    k_frame_stats<1><<<grid, STATS_THREADS, smem, stream>>>(g, d_frames, d_out_index, n, d_stats, d_rowsum, d_colsum);
+    k_frame_stats<1><<<grid, STATS_THREADS, smem, stream>>>(g, d_frames, n, d_stats, d_rowsum, d_colsum);
     ctx->launches += 2;
     EPID_CUDA(cudaGetLastError());
     return EPID_OK;

@@ -39,9 +39,9 @@ struct FrameStats {  // per frame, device memory
 int make_stats_geom(StatsGeom* g, int H, int W);
 
 // Launches the fast (packed-u16) pass for frames d_frames[0..n) and the exact fallback for frames that overflowed.
-// out_index == nullptr: frame i writes slot i.  rowsum: [slot][H] u32, colsum: [slot][W] u32 (may be null).
+// rowsum: [n][H] u32, colsum: [n][W] u32 (may be null).
 int launch_frame_stats(epid_ctx* ctx, cudaStream_t stream, const StatsGeom& g, const FrameRef* d_frames,
-                       const int* d_out_index, int n, FrameStats* d_stats, uint32_t* d_rowsum, uint32_t* d_colsum);
+                       int n, FrameStats* d_stats, uint32_t* d_rowsum, uint32_t* d_colsum);
 // check_inversion_by_histogram statistics (three percentile pairs in g.ranks): min / max / sum / row / column sums exactly; the decision
 // certified from exact counts (FrameStats.overflow = 2 + inverted) or, where the bounds overlap, exact order statistics (overflow = 0)
 int launch_frame_stats_inversion(epid_ctx* ctx, cudaStream_t stream, const StatsGeom& g, const FrameRef* d_frames, int n, FrameStats* d_stats,

@@ -282,7 +282,7 @@ def test_pf_degenerate_inputs_fail_like_the_reference():
         pf.analyze_batch(np.zeros((1, 1024, 1024), np.float32), 2.56)
 
 
-def _leafband_cases():
+def _window_cases():
     from oracle import synth
     from tests.golden import pf_docs_cases as dc
 
@@ -307,49 +307,6 @@ def _leafband_cases():
         fr, ps, sid, ak = dc.docs_frame(nm)
         out["docs_" + nm] = (fr[None], (1 / ps) * sid / 1000.0, ak)
     return out
-
-
-@pytest.mark.parametrize("name", list(_leafband_cases()))
-def test_leafband_kernel_equals_per_window_kernel(name):
-    """The experimental leaf-band window kernel (one CTA per leaf, all pickets at once; opt-in, see DESIGN.md 4.6) must reproduce
-    the per-window kernel bit for bit."""
-    from pylinac_b200 import _native as nat
-    from pylinac_b200 import picketfence as pf
-
-    frames, dpmm, kw = _leafband_cases()[name]
-    ctx = nat.Context.default()
-    try:
-        ctx.set_option(nat.OPT_PF_LEAFBAND, 0)
-        old = pf.analyze_batch(frames, dpmm, **kw)
-        ctx.set_option(nat.OPT_PF_LEAFBAND, 1)
-        new = pf.analyze_batch(frames, dpmm, **kw)
-    finally:
-        ctx.set_option(nat.OPT_PF_LEAFBAND, 0)
-    for k in old.summary.dtype.names:
-        np.testing.assert_array_equal(old.summary[k], new.summary[k], err_msg=k)
-    for i in range(len(frames)):
-        if int(old.summary["status"][i]) == 0:
-            m = int(old.summary["n_meas"][i])
-            assert m > 0
-            for k in old.meas.dtype.names:
-                np.testing.assert_array_equal(old.meas[k][i, :m], new.meas[k][i, :m], err_msg=k)
-
-
-def test_leafband_kernel_runs_when_enabled():
-    from oracle import synth
-    from pylinac_b200 import _native as nat
-    from pylinac_b200 import picketfence as pf
-
-    ctx = nat.Context.default()
-    frames = np.stack([synth.bench_pf_frame(i) for i in range(60, 76)])
-    b = nat.Batch.upload(ctx, frames)
-    try:
-        ctx.set_option(nat.OPT_PF_LEAFBAND, 1)
-        st = nat.pf_bench_stages(ctx, b, pf.make_params(2.56, frames.shape[1:]), 2)
-    finally:
-        ctx.set_option(nat.OPT_PF_LEAFBAND, 0)
-        b.free()
-    assert st["k_pf_leafband"] > 5 * st["k_pf_windows_fast"] > 0
 
 
 def test_pf_host_pipeline_staged_and_direct_result_paths_agree():
@@ -380,14 +337,14 @@ def test_pf_host_pipeline_staged_and_direct_result_paths_agree():
             np.testing.assert_array_equal(m_direct[k][i, :m], m_staged[k][i, :m], err_msg=k)
 
 
-@pytest.mark.parametrize("name", list(_leafband_cases()))
+@pytest.mark.parametrize("name", list(_window_cases()))
 def test_two_kernel_window_path_equals_per_window_kernel(name):
     """The default window path (k_pf_win_medians + k_pf_win_fwxm, pf_windows2.cu) must reproduce the single per-window kernel
     (k_pf_windows_fast, pinned to the reference by the golden tests) bit for bit, on frames it covers and on frames it declines."""
     from pylinac_b200 import _native as nat
     from pylinac_b200 import picketfence as pf
 
-    frames, dpmm, kw = _leafband_cases()[name]
+    frames, dpmm, kw = _window_cases()[name]
     ctx = nat.Context.default()
     try:
         ctx.set_option(nat.OPT_PF_WIN2, 0)
@@ -419,6 +376,18 @@ def test_two_kernel_window_path_runs_for_the_benchmark_frames():
     finally:
         b.free()
     assert st["k_pf_win_medians"] > 5 * st["k_pf_windows_fast"] > 0, st
+    # every kernel of the default pipeline is charged to its own stage, and only those
+    assert {k for k, v in st.items() if v > 0} == {"k_pf_init + k_pf_pilot", "k_pf_stream", "k_pf_tail", "k_pf_windows_fast",
+                                                   "k_pf_windows (generic)", "k_pf_finalize", "k_pf_win_medians", "k_pf_win_fwxm"}, st
+
+
+def test_retired_pf_options_are_rejected():
+    from pylinac_b200 import _native as nat
+
+    ctx = nat.Context.default()
+    for key in (2, 4, 6):       # retired option keys
+        with pytest.raises(ValueError):
+            ctx.set_option(key, 1)
 
 
 def test_pf_mixed_batch_matches_the_oracle_frame_by_frame():
@@ -516,11 +485,11 @@ def _assert_same_results(a, b):
             np.testing.assert_array_equal(ma[k][i, :m], mb[k][i, :m], err_msg=f"{k} frame {i}")
 
 
-def test_pf_certified_noise_rerun_equals_the_exact_rerun_and_overlaps():
+def test_pf_certified_noise_rerun_equals_the_exact_rerun():
     """The per-frame fallback: frames whose _has_noise() the single exact count certifies are median filtered and re-run by the
     certified fast pipeline (frames with a hot block are deferred again -> exact pipeline).  Every variant -- fast / exact re-run,
-    overlapped on the second stream or serial, device-resident or host entry point -- must return bit-identical rows, and the hot-pixel
-    frames must equal the oracle."""
+    device-resident (overlapped with the batch on the second stream) or host entry point -- must return bit-identical rows, and the
+    hot-pixel frames must equal the oracle."""
     from oracle import pf_oracle
     from pylinac_b200 import _native as nat
     from pylinac_b200 import picketfence as pf
@@ -533,24 +502,20 @@ def test_pf_certified_noise_rerun_equals_the_exact_rerun_and_overlaps():
     counts = {}
     try:
         for fast_redo in (1, 0):
-            for overlap in (1, 0):
-                ctx.set_option(nat.OPT_PF_FAST_REDO, fast_redo)
-                ctx.set_option(nat.OPT_PF_OVERLAP_REDO, overlap)
-                r0, e0 = ctx.counter(nat.CTR_PF_REDONE_FRAMES), ctx.counter(nat.CTR_PF_EXACT_FRAMES)
-                results[(fast_redo, overlap, "dev")] = nat.pf_analyze(ctx, b, params)
-                counts[(fast_redo, overlap)] = (ctx.counter(nat.CTR_PF_REDONE_FRAMES) - r0, ctx.counter(nat.CTR_PF_EXACT_FRAMES) - e0)
-                s, m = nat.pf_analyze(ctx, frames, params)
-                results[(fast_redo, overlap, "host")] = (s.copy(), m.copy())
+            ctx.set_option(nat.OPT_PF_FAST_REDO, fast_redo)
+            r0, e0 = ctx.counter(nat.CTR_PF_REDONE_FRAMES), ctx.counter(nat.CTR_PF_EXACT_FRAMES)
+            results[(fast_redo, "dev")] = nat.pf_analyze(ctx, b, params)
+            counts[fast_redo] = (ctx.counter(nat.CTR_PF_REDONE_FRAMES) - r0, ctx.counter(nat.CTR_PF_EXACT_FRAMES) - e0)
+            s, m = nat.pf_analyze(ctx, frames, params)
+            results[(fast_redo, "host")] = (s.copy(), m.copy())
     finally:
         ctx.set_option(nat.OPT_PF_FAST_REDO, 1)
-        ctx.set_option(nat.OPT_PF_OVERLAP_REDO, 1)
         b.free()
     n_hot, n_block = kinds.count("hot"), kinds.count("block")
     assert n_hot >= 8 and n_block >= 4
-    for overlap in (1, 0):
-        assert counts[(1, overlap)] == (n_hot + n_block, n_block), counts      # only the hot-block frames need the exact pipeline
-        assert counts[(0, overlap)] == (n_hot + n_block, n_hot + n_block), counts
-    ref = results[(0, 0, "dev")]
+    assert counts[1] == (n_hot + n_block, n_block), counts      # only the hot-block frames need the exact pipeline
+    assert counts[0] == (n_hot + n_block, n_hot + n_block), counts
+    ref = results[(0, "dev")]
     for key, val in results.items():
         _assert_same_results(ref, val)
     s, m = ref

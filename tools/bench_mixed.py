@@ -23,13 +23,12 @@ for i in rng.choice(n, n // 20, replace=False):
     f.ravel()[rng.integers(0, f.size, 40)] = 65535
     mixed[i] = f
 mb = nat.Batch.upload(ctx, mixed)
-for fast_redo, overlap in ((0, 0), (1, 0), (0, 1), (1, 1)):
+for fast_redo in (0, 1):
     ctx.set_option(nat.OPT_PF_FAST_REDO, fast_redo)
-    ctx.set_option(nat.OPT_PF_OVERLAP_REDO, overlap)
     nat.pf_bench_timed(ctx, mb, params, 2)
     for rep in range(3):
         e0 = ctx.counter(nat.CTR_PF_EXACT_FRAMES)
         t, st, l, r = nat.pf_bench_timed(ctx, mb, params, 10)
-        print(f"mixed fast_redo={fast_redo} overlap={overlap}: {t / 10:.3f} ms/step, launches {l / 10:.0f}, redone/step {r / 10:.0f}, "
+        print(f"mixed fast_redo={fast_redo}: {t / 10:.3f} ms/step, launches {l / 10:.0f}, redone/step {r / 10:.0f}, "
               f"exact/step {(ctx.counter(nat.CTR_PF_EXACT_FRAMES) - e0) / 10:.0f}; stages(us): " +
               ", ".join(f"{k.split(' ')[0]} {v * 1e3:.0f}" for k, v in st.items() if v > 0))

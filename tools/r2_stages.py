@@ -39,7 +39,7 @@ def main():
     nat.pf_bench(ctx, b, params, 3)
     total, stream_ms, launches = nat.pf_bench(ctx, b, params, a.iters)
     st = nat.pf_bench_stages(ctx, b, params, a.iters)
-    out = {"frames": a.frames, "win2": a.win2, "mixed_pct": a.mixed, "wa_grid": os.environ.get("EPID_WA_GRID"), "ms_per_step": total / a.iters,
+    out = {"frames": a.frames, "win2": a.win2, "mixed_pct": a.mixed, "ms_per_step": total / a.iters,
            "fps": a.frames * a.iters / (total * 1e-3), "launches_per_step": launches / a.iters,
            "redone": ctx.counter(nat.CTR_PF_REDONE_FRAMES), "stages_ms": {k: round(v, 4) for k, v in st.items() if v > 0}}
     print(json.dumps(out))
