@@ -31,7 +31,8 @@ enum {
     EPID_ERR_INVALID = -3,        /* bad argument (maps to ValueError) */
     EPID_ERR_UNSUPPORTED = -4,    /* size / dtype outside what the kernels support */
     EPID_ERR_NOMEM = -5,
-    EPID_ERR_NCCL = -6
+    EPID_ERR_NCCL = -6,
+    EPID_ERR_INDEX = -7           /* an index outside the array, as numpy's IndexError (disk ROIs over the bottom / right edge) */
 };
 
 /* element types of image batches (numpy dtypes the reference's operators preserve, core/array_utils.py) */
@@ -504,6 +505,26 @@ int32_t epid_gamma(epid_ctx* ctx, const epid_batch* ref, const epid_batch* comp,
  * evaluated on every frame of the batch: outputs [n][nroi] (may be NULL).  std is the population standard deviation (np.std). */
 int32_t epid_roi_stats(epid_ctx* ctx, const epid_batch* b, int32_t nroi, const double* verts_xy, double* count, double* mean,
                        double* std, double* mn, double* mx);
+/* DiskROI.pixel_value / mean / std / min / max (core/roi.py:103-132) and LowContrastDiskROI.percentile (core/roi.py:406-408) of ndisk
+ * disks (centers_xy[ndisk][(x, y)], radii[ndisk]) on every frame: outputs [n][ndisk] (may be NULL), pct [n][ndisk][npct] (may be NULL).
+ * Pixel set: skimage.draw.disk(center=(y, x), radius) WITHOUT shape, as DiskROI.circle_mask (core/roi.py:134-138) calls it -- box
+ * ceil(c - r) .. floor(c + r), ((i - r_org) / r)**2 + ((j - c_org) / r)**2 < 1 in fp64, and numpy's negative-index wrap-around for rows /
+ * columns in [-dim, -1].  A selected index outside [-dim, dim - 1] returns EPID_ERR_INDEX.  8 / 16-bit frames: exact integer moments
+ * (mean, min, max bit-exact, std from the exact N * S2 - S1^2); other dtypes: fp64 moments, std from the centred second moment.
+ * median (np.median) and the percentiles (np.percentile, linear; 0 <= p <= 100 else EPID_ERR_INVALID; at most EPID_DISK_MAX_PCT) are
+ * exact order statistics (radix select) combined with numpy's arithmetic (float32 frames in float32).  A disk with no pixels gives
+ * count 0 and NaN statistics; a disk containing a NaN pixel gives NaN statistics. */
+#define EPID_DISK_MAX_PCT 16
+int32_t epid_disk_roi_stats(epid_ctx* ctx, const epid_batch* b, int32_t ndisk, const double* centers_xy, const double* radii,
+                            int32_t npct, const double* percentiles, double* count, double* mean, double* std, double* mn,
+                            double* mx, double* median, double* pct);
+/* DiskROI.circle_mask / pixel_values (clip = 0, core/roi.py:103-105, 134-138) and the pixel set of masked_array (clip = 1:
+ * draw.disk(..., shape=shape), core/roi.py:140-150) of one disk on frame `frame`: *count = number of pixels; when values != NULL
+ * (capacity >= count, element type = the batch dtype) the values in np.nonzero (row-major) order, and when rows / cols != NULL the row /
+ * column indices skimage returns (unwrapped: negative for the wrapped rows / columns of clip = 0).  Call once with values == NULL for
+ * the count, then with a buffer.  clip = 0 and a selected index outside [-dim, dim - 1]: EPID_ERR_INDEX. */
+int32_t epid_disk_roi_pixels(epid_ctx* ctx, const epid_batch* b, int32_t frame, const double* center_xy, double radius, int32_t clip,
+                             int64_t capacity, void* values, int32_t* rows, int32_t* cols, int64_t* count);
 /* WeightedCentroid.calculate (metrics/image.py:959-983): cx = sum(x * a) / sum(a), cy likewise; total = sum(a) (may be NULL). */
 int32_t epid_weighted_centroid(epid_ctx* ctx, const epid_batch* b, double* cx, double* cy, double* total);
 

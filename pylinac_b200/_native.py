@@ -16,7 +16,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("EPID_LIB") or os.path.join(_HERE, "libepid.so")      # EPID_LIB: kernel-variant experiments (tools/)
 
 EPID_OK = 0
-ERR_NO_DEVICE, ERR_CUDA, ERR_INVALID, ERR_UNSUPPORTED, ERR_NOMEM, ERR_NCCL = -1, -2, -3, -4, -5, -6
+ERR_NO_DEVICE, ERR_CUDA, ERR_INVALID, ERR_UNSUPPORTED, ERR_NOMEM, ERR_NCCL, ERR_INDEX = -1, -2, -3, -4, -5, -6, -7
 
 U8, U16, I32, F32, F64, I16, I64 = 0, 1, 2, 3, 4, 5, 6
 _NP2DT = {np.dtype(np.uint8): U8, np.dtype(np.uint16): U16, np.dtype(np.int32): I32, np.dtype(np.float32): F32,
@@ -313,6 +313,8 @@ _SIGNATURES = {
     "epid_gamma": [_P, _P, _P, C.c_double, C.c_double, C.c_double, C.POINTER(_P)],
     "epid_disk_locate": [_P, _P, _P, _P],
     "epid_roi_stats": [_P, _P, C.c_int32, _P, _P, _P, _P, _P, _P],
+    "epid_disk_roi_stats": [_P, _P, C.c_int32, _P, _P, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P],
+    "epid_disk_roi_pixels": [_P, _P, C.c_int32, _P, C.c_double, C.c_int32, C.c_int64, _P, _P, _P, C.POINTER(C.c_int64)],
     "epid_weighted_centroid": [_P, _P, _P, _P, _P],
     "epid_vmat_analyze": [_P, _P, _P, C.POINTER(VmatParams), _P],
     "epid_divide": [_P, _P, _P, _P, C.POINTER(_P)],
@@ -364,6 +366,8 @@ def check(rc):
             raise NoDeviceError(rc, msg)
         if rc == ERR_INVALID:
             raise ValueError(msg)
+        if rc == ERR_INDEX:
+            raise IndexError(msg)
         raise NativeError(rc, msg)
 
 
@@ -777,6 +781,52 @@ def roi_stats(ctx: Context, frames, verts_xy) -> dict:
         if own:
             b.free()
     return out
+
+
+DISK_MAX_PCT = 16
+
+
+def disk_roi_stats(ctx: Context, frames, centers_xy, radii, percentiles=()) -> dict:
+    """DiskROI statistics of k disks (centers_xy [k, 2] as (x, y), radii [k]) on every frame -> dict of [n, k] arrays (count, mean, std,
+    min, max, median) and "percentile" [n, k, p].  Empty disks give count 0 and NaN; IndexError for a disk over the bottom / right edge."""
+    c = np.ascontiguousarray(centers_xy, dtype=np.float64).reshape(-1, 2)
+    r = np.ascontiguousarray(np.broadcast_to(np.asarray(radii, dtype=np.float64), (len(c),)))
+    q = np.ascontiguousarray([float(p) for p in np.atleast_1d(percentiles)], dtype=np.float64)
+    if len(q) > DISK_MAX_PCT:
+        raise ValueError(f"at most {DISK_MAX_PCT} percentiles per call")
+    b, own = _as_batch(ctx, frames)
+    (n, _, _), _ = b.shape_dtype
+    out = {k: np.empty((n, len(c))) for k in ("count", "mean", "std", "min", "max", "median")}
+    out["percentile"] = np.empty((n, len(c), len(q)))
+    try:
+        check(lib().epid_disk_roi_stats(ctx.handle, b.handle, len(c), _ptr(c), _ptr(r), len(q), _ptr(q) if len(q) else None,
+                                        _ptr(out["count"]), _ptr(out["mean"]), _ptr(out["std"]), _ptr(out["min"]), _ptr(out["max"]),
+                                        _ptr(out["median"]), _ptr(out["percentile"])))
+    finally:
+        if own:
+            b.free()
+    return out
+
+
+def disk_roi_pixels(ctx: Context, frames, frame: int, center_xy, radius: float, clip: bool = False, indices: bool = False):
+    """One disk's pixel values on frame ``frame`` in np.nonzero order (DiskROI.circle_mask; clip=True: the clipped pixel set of
+    masked_array).  indices=True also returns skimage's (rows, cols)."""
+    c = np.ascontiguousarray(center_xy, dtype=np.float64).reshape(2)
+    b, own = _as_batch(ctx, frames)
+    try:
+        _, dt = b.shape_dtype
+        n = C.c_int64()
+        check(lib().epid_disk_roi_pixels(ctx.handle, b.handle, int(frame), _ptr(c), float(radius), int(bool(clip)), 0, None, None, None,
+                                         C.byref(n)))
+        vals = np.empty(n.value, dt)
+        rows, cols = np.empty(n.value, np.int32), np.empty(n.value, np.int32)
+        if n.value:
+            check(lib().epid_disk_roi_pixels(ctx.handle, b.handle, int(frame), _ptr(c), float(radius), int(bool(clip)), n.value, _ptr(vals),
+                                             _ptr(rows), _ptr(cols), C.byref(n)))
+    finally:
+        if own:
+            b.free()
+    return (vals, rows.astype(np.intp), cols.astype(np.intp)) if indices else vals
 
 
 def vmat_analyze(ctx: Context, img1, img2, params: VmatParams) -> np.ndarray:

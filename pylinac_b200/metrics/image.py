@@ -1,5 +1,6 @@
-"""2-D image metric plug-ins -- mirror of ``pylinac.metrics.image`` (metrics/image.py:38-76, 402-667, 959-983): ``MetricBase``,
-``SizedDiskRegion`` / ``SizedDiskLocator`` (the BB finder) and ``WeightedCentroid``, computed through ``image.compute(metric)``.
+"""2-D image metric plug-ins -- mirror of ``pylinac.metrics.image`` (metrics/image.py:38-272, 402-667, 959-983): ``MetricBase``,
+``DiskROIMetric`` / ``RectangleROIMetric`` (ROI samplers), ``SizedDiskRegion`` / ``SizedDiskLocator`` (the BB finder) and
+``WeightedCentroid``, computed through ``image.compute(metric)``.
 
 The pixel work runs on the device: the disk locator is the threshold sweep / labelling / region-property kernel of the
 Winston-Lutz pipeline exposed on its own (``epid_disk_locate``, csrc/wl.cu), the weighted centroid is a device reduction
@@ -16,6 +17,7 @@ import numpy as np
 
 from .. import _native as nat
 from ..core.geometry import Point
+from ..core.roi import DiskROI, RectangleROI
 from .features import DEFAULT_CONDITIONS, conditions_mask
 
 
@@ -52,6 +54,65 @@ class MetricBase(ABC):
 
     def additional_plots(self):
         pass
+
+
+class DiskROIMetric(MetricBase):
+    """Samples a disk ROI of the image -> ``DiskROI`` (metrics/image.py:98-177).  ``from_physical`` takes mm; like the reference,
+    ``calculate()`` scales the radius and the centre by dpmm IN PLACE every time it runs (:159-161)."""
+
+    roi: DiskROI
+    _from_physical: bool = False
+
+    @classmethod
+    def from_physical(cls, radius_mm: float, center_mm: Point, name: str = "Disk ROI Metric", edgecolor: str = "b", **kwargs):
+        instance = cls(radius_mm, center_mm, name, edgecolor, **kwargs)
+        instance._from_physical = True
+        return instance
+
+    def __init__(self, radius: float, center: Point, name: str = "Disk ROI Metric", edgecolor: str = "b", **kwargs):
+        self.radius = radius
+        self.center = center
+        self.name = name
+        self.edge_color = edgecolor
+        self.kwargs = kwargs
+
+    def calculate(self) -> DiskROI:
+        if self._from_physical:
+            self.radius *= self.image.dpmm
+            self.center *= self.image.dpmm
+        self.roi = DiskROI(array=self.image.array, center=self.center, radius=self.radius)
+        return self.roi
+
+
+class RectangleROIMetric(MetricBase):
+    """Samples a rectangle ROI of the image -> ``RectangleROI`` (metrics/image.py:180-272); ``from_physical`` scales width, height and
+    centre by dpmm in place on every ``calculate()`` (:246-250), as the reference does."""
+
+    roi: RectangleROI
+    _from_physical: bool = False
+
+    @classmethod
+    def from_physical(cls, width_mm: float, height_mm: float, center_mm: Point, name: str = "Rectangle ROI Metric", edgecolor: str = "b",
+                      **kwargs):
+        instance = cls(width_mm, height_mm, center_mm, name, edgecolor, **kwargs)
+        instance._from_physical = True
+        return instance
+
+    def __init__(self, width: float, height: float, center: Point, name: str = "Rectangle ROI Metric", edgecolor: str = "b", **kwargs):
+        self.height = height
+        self.width = width
+        self.center = center
+        self.name = name
+        self.edge_color = edgecolor
+        self.kwargs = kwargs
+
+    def calculate(self) -> RectangleROI:
+        if self._from_physical:
+            self.width *= self.image.dpmm
+            self.height *= self.image.dpmm
+            self.center *= self.image.dpmm
+        self.roi = RectangleROI(array=self.image.array, center=self.center, width=self.width, height=self.height)
+        return self.roi
 
 
 class DiskRegion:
